@@ -62,6 +62,9 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-tf32", action="store_true", help="skip the secondary plain-tf32 measurement")
     ap.add_argument("--curve", action="store_true", help="(kept for compatibility: the curve is always printed)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed rounds, write what the last one computed (every node's model, the round's "
+                         "evaluation) to DIR/<name>.npy, to compare two builds output for output")
     return ap.parse_args()
 
 
@@ -272,6 +275,23 @@ def time_rounds(sim, rounds: int, world: int, resume: bool = True):
     return start.elapsed_time(stop)
 
 
+def dump_outputs(sim, rep, out_dir: str, rank: int, world: int):
+    """What the timed rounds hand back to a caller, as of the last one: every node's model (its parameters, flattened
+    in module order; with several GPUs each rank writes the nodes it holds) and that round's evaluation (mean over
+    the nodes)."""
+    import numpy as np
+    import torch
+    from gossipy_b200.parallel import runtime as prt
+    os.makedirs(out_dir, exist_ok=True)
+    ids = [i for i in sorted(sim.nodes) if world == 1 or prt.is_mine(i)]
+    rows = torch.stack([torch.cat([p.detach().reshape(-1) for p in sim.nodes[i].model_handler.model.parameters()])
+                        for i in ids]).float().cpu()
+    np.save(os.path.join(out_dir, "models%s.npy" % ("" if world == 1 else "_rank%d" % rank)), rows.numpy())
+    if rank == 0:
+        for name, v in rep.get_evaluation(False)[-1][1].items():
+            np.save(os.path.join(out_dir, "eval_%s.npy" % name), np.array([float(v)], dtype=np.float64))
+
+
 def run_native(args, rank, world):
     import torch
     from gossipy_b200 import ops
@@ -283,6 +303,8 @@ def run_native(args, rank, world):
     launches0 = ops.launch_count
     with ClockSampler(torch.cuda.current_device() if torch.cuda.is_available() else 0) as clk:
         ms = time_rounds(sim, K, world)
+    if args.dump_outputs:
+        dump_outputs(sim, rep, args.dump_outputs, rank, world)
     launches = int(sum_over_ranks(ops.launch_count - launches0, world))
     ms = max_over_ranks(ms, world)
     value = K / (ms / 1e3)
@@ -444,6 +466,8 @@ def run_reference(args, rank, world):
 
 def main():
     args = parse()
+    if args.dump_outputs and args.impl != "native":
+        sys.exit("--dump-outputs writes the outputs of this framework's rounds (--impl native)")
     rank, world, _ = dist_setup(args.gpus)
     try:
         if args.impl == "reference":

@@ -1,4 +1,6 @@
-"""Test configuration: the ``gpu`` marker, reference import shims and state isolation."""
+"""Test configuration: the ``gpu`` marker, state isolation, and the original gossipy's side of the comparisons
+(recorded results, or the original itself with its import shims)."""
+import json
 import os
 import sys
 import types
@@ -40,8 +42,8 @@ def _fresh_state():
 
 def _import_reference():
     """Import the read-only reference with the three environment shims of SURVEY §0."""
-    ref_root = "/root/reference"
-    if not os.path.isdir(os.path.join(ref_root, "gossipy")):
+    ref_root = os.environ.get("GOSSIPY_REFERENCE", "")
+    if not ref_root or not os.path.isdir(os.path.join(ref_root, "gossipy")):
         return None
     for name in ("matplotlib", "matplotlib.pyplot", "pyparsing"):
         if name not in sys.modules:
@@ -75,9 +77,85 @@ def _import_reference():
         return None
 
 
-@pytest.fixture(scope="session")
-def ref():
-    mod = _import_reference()
-    if mod is None:
-        pytest.skip("reference not importable")
-    return mod
+GOLDEN = os.path.join(ROOT, "tests", "golden", "reference")
+_golden = {}        # test module file name -> {result key: encoded value}
+_recorded = set()   # files holding results recorded in this session
+
+
+def _encode(v):
+    import torch
+    if isinstance(v, torch.Tensor):
+        t = v.detach().cpu()
+        return {"__tensor__": str(t.dtype).replace("torch.", ""), "shape": list(t.shape), "data": t.reshape(-1).tolist()}
+    if isinstance(v, np.ndarray):
+        return {"__ndarray__": v.dtype.str, "shape": list(v.shape), "data": v.reshape(-1).tolist()}
+    if isinstance(v, np.generic):
+        return v.item()
+    if isinstance(v, dict):
+        return {"__dict__": [[_encode(k), _encode(x)] for k, x in v.items()]}
+    if isinstance(v, (list, tuple)):
+        return [_encode(x) for x in v]
+    assert v is None or isinstance(v, (bool, int, float, str)), type(v)
+    return v
+
+
+def _decode(v):
+    import torch
+    if isinstance(v, list):
+        return [_decode(x) for x in v]
+    if isinstance(v, dict):
+        if "__tensor__" in v:
+            return torch.tensor(v["data"], dtype=getattr(torch, v["__tensor__"])).reshape(v["shape"])
+        if "__ndarray__" in v:
+            return np.array(v["data"], dtype=np.dtype(v["__ndarray__"])).reshape(v["shape"])
+        return {_decode_key(k): _decode(x) for k, x in v["__dict__"]}
+    return v
+
+
+def _decode_key(k):
+    return tuple(_decode_key(x) for x in k) if isinstance(k, list) else k
+
+
+class Reference:
+    """Results of the original gossipy for one test.
+
+    ``ref(fn)`` returns ``fn(gossipy)``.  With ``GOSSIPY_REFERENCE`` naming a checkout of the original project the
+    function runs against it and its result is recorded under ``tests/golden/reference/``; without it, the result
+    recorded there is returned, so every comparison with the original runs on any machine.  Results are keyed by the
+    test id and the order of the calls within the test; values are numbers, strings, lists, tuples (read back as
+    lists), dicts, tensors and arrays (read back with their dtype, exactly)."""
+
+    def __init__(self, module, nodeid):
+        path, _, name = nodeid.partition("::")
+        self.module, self.file, self.name, self.calls = module, os.path.basename(path)[:-3] + ".json", name, 0
+        if self.file not in _golden:
+            try:
+                with open(os.path.join(GOLDEN, self.file)) as f:
+                    _golden[self.file] = json.load(f)
+            except FileNotFoundError:
+                _golden[self.file] = {}
+
+    def __call__(self, fn):
+        key = "%s#%d" % (self.name, self.calls)
+        self.calls += 1
+        store = _golden[self.file]
+        if self.module is not None:
+            store[key] = _encode(fn(self.module))
+            _recorded.add(self.file)
+        elif key not in store:
+            pytest.fail("no recorded result of the original gossipy for %s in %s (record it: GOSSIPY_REFERENCE=<checkout> "
+                        "pytest ...)" % (key, os.path.join(GOLDEN, self.file)))
+        return _decode(store[key])
+
+
+def pytest_sessionfinish(session):
+    for name in sorted(_recorded):
+        os.makedirs(GOLDEN, exist_ok=True)
+        with open(os.path.join(GOLDEN, name), "w") as f:
+            json.dump(_golden[name], f, sort_keys=True, separators=(",", ":"))
+            f.write("\n")
+
+
+@pytest.fixture
+def ref(request):
+    return Reference(_import_reference(), request.node.nodeid)

@@ -34,21 +34,48 @@ def _params(fn):
     return [p for p in sig.parameters.values() if p.name != "self"]
 
 
-def _check_callable(ref_fn, our_fn, where):
-    rp, op = _params(ref_fn), _params(our_fn)
+def _describe_callable(fn):
+    params = _params(fn)
+    return None if params is None else [(p.name, p.kind.name, p.default is not p.empty) for p in params]
+
+
+def _describe_module(rmod, extra):
+    """The reference module's public API as plain data: names, kinds, parameters, class members."""
+    names = list(getattr(rmod, "__all__", [])) + [n for n in extra if hasattr(rmod, n)]
+    out = []
+    for name in dict.fromkeys(names):
+        robj = getattr(rmod, name)
+        if inspect.isclass(robj):
+            d = {"kind": "class", "skip": issubclass(robj, BaseException) or name in ("LOG",), "members": []}
+            if "__init__" in vars(robj):
+                d["init"] = _describe_callable(robj.__init__)
+            for attr, member in vars(robj).items():
+                if attr.startswith("_") or inspect.isclass(member) or inspect.ismodule(member):
+                    continue       # (the reference imports a class inside one class body)
+                d["members"].append((attr, _describe_callable(member) if inspect.isfunction(member) else False))
+        elif inspect.isfunction(robj):
+            d = {"kind": "function", "params": _describe_callable(robj)}
+        else:
+            d = {"kind": "other"}
+        out.append((name, d))
+    return out
+
+
+def _check_callable(rp, our_fn, where):
+    op = _params(our_fn)
     if rp is None or op is None:
         return
     if any(p.kind in (p.VAR_POSITIONAL, p.VAR_KEYWORD) for p in op):
         return      # we forward *args/**kwargs (e.g. handler subclasses): accepted by construction
     ours = [p.name for p in op]
-    for i, p in enumerate(rp):
-        if p.kind in (p.VAR_POSITIONAL, p.VAR_KEYWORD):
+    for i, (name, kind, has_default) in enumerate(rp):
+        if kind in ("VAR_POSITIONAL", "VAR_KEYWORD"):
             continue
-        assert p.name in ours, "%s: parameter %r missing (ours: %s)" % (where, p.name, ours)
-        if p.kind == p.POSITIONAL_OR_KEYWORD and p.default is p.empty:
-            assert ours.index(p.name) == i, "%s: positional parameter %r moved" % (where, p.name)
+        assert name in ours, "%s: parameter %r missing (ours: %s)" % (where, name, ours)
+        if kind == "POSITIONAL_OR_KEYWORD" and not has_default:
+            assert ours.index(name) == i, "%s: positional parameter %r moved" % (where, name)
     for p in op:      # anything we added must be optional
-        if p.name not in [q.name for q in rp]:
+        if p.name not in [q[0] for q in rp]:
             assert p.default is not p.empty or p.kind == p.KEYWORD_ONLY and p.default is not p.empty, \
                 "%s: new required parameter %r" % (where, p.name)
 
@@ -56,32 +83,30 @@ def _check_callable(ref_fn, our_fn, where):
 @pytest.mark.parametrize("ref_name", sorted(MODULES))
 def test_module_api_parity(ref, ref_name):
     ours_name, extra = MODULES[ref_name]
-    rmod = importlib.import_module(ref_name)
+    api = ref(lambda rg: _describe_module(importlib.import_module(ref_name), extra))
     omod = importlib.import_module(ours_name)
-    names = list(getattr(rmod, "__all__", [])) + [n for n in extra if hasattr(rmod, n)]
-    assert names, ref_name
-    for name in dict.fromkeys(names):
+    assert api, ref_name
+    for name, d in api:
         assert hasattr(omod, name), "%s.%s is missing" % (ours_name, name)
-        robj, oobj = getattr(rmod, name), getattr(omod, name)
-        if inspect.isclass(robj):
+        oobj = getattr(omod, name)
+        if d["kind"] == "class":
             assert inspect.isclass(oobj), name
-            if issubclass(robj, BaseException) or name in ("LOG",):
+            if d["skip"]:
                 continue
-            if "__init__" in vars(robj):
-                _check_callable(robj.__init__, oobj.__init__, "%s.%s.__init__" % (ours_name, name))
-            for attr, member in vars(robj).items():
-                if attr.startswith("_") or inspect.isclass(member) or inspect.ismodule(member):
-                    continue       # (the reference imports a class inside one class body)
+            if "init" in d:
+                _check_callable(d["init"], oobj.__init__, "%s.%s.__init__" % (ours_name, name))
+            for attr, params in d["members"]:
                 assert hasattr(oobj, attr), "%s.%s.%s is missing" % (ours_name, name, attr)
-                if inspect.isfunction(member):
-                    _check_callable(member, getattr(oobj, attr), "%s.%s.%s" % (ours_name, name, attr))
-        elif inspect.isfunction(robj):
-            _check_callable(robj, oobj, "%s.%s" % (ours_name, name))
+                if params is not False:
+                    _check_callable(params, getattr(oobj, attr), "%s.%s.%s" % (ours_name, name, attr))
+        elif d["kind"] == "function":
+            _check_callable(d["params"], oobj, "%s.%s" % (ours_name, name))
+
+
+def _enum_members(core):
+    return [[(m.name, m.value) for m in getattr(core, name)] for name in ("CreateModelMode", "AntiEntropyProtocol", "MessageType")]
 
 
 def test_enum_members_match(ref):
-    import gossipy.core as rc
     import gossipy_b200.core as oc
-    for name in ("CreateModelMode", "AntiEntropyProtocol", "MessageType"):
-        r, o = getattr(rc, name), getattr(oc, name)
-        assert [(m.name, m.value) for m in r] == [(m.name, m.value) for m in o]
+    assert [[tuple(m) for m in e] for e in ref(lambda rg: _enum_members(rg.core))] == _enum_members(oc)

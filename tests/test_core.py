@@ -17,11 +17,13 @@ def _ring(n):
     return A
 
 
+def _enums(core):
+    return {name: {m.name: m.value for m in getattr(core, name)}
+            for name in ("CreateModelMode", "AntiEntropyProtocol", "MessageType")}
+
+
 def test_enums_match_reference(ref):
-    import gossipy.core as rc
-    for name in ("CreateModelMode", "AntiEntropyProtocol", "MessageType"):
-        ours, theirs = getattr(g.core, name), getattr(rc, name)
-        assert {m.name: m.value for m in ours} == {m.name: m.value for m in theirs}
+    assert _enums(g.core) == ref(lambda rg: _enums(rg.core))
 
 
 def test_message_size_rules():
@@ -59,14 +61,18 @@ def test_delays():
 
 
 def test_topology_degrees_fix_and_compat(ref):
-    import gossipy.core as rc
     A = _ring(6)
-    ours, theirs = StaticP2PNetwork(6, A), rc.StaticP2PNetwork(6, A)
+
+    def theirs(rg):
+        net = rg.core.StaticP2PNetwork(6, A)
+        return [[int(x) for x in net.get_peers(i)] for i in range(6)], net.size(0)
+    peers, size0 = ref(theirs)
+    ours = StaticP2PNetwork(6, A)
     for i in range(6):
-        assert list(ours.get_peers(i)) == [int(x) for x in theirs.get_peers(i)]
+        assert list(ours.get_peers(i)) == peers[i]
     assert ours.size() == 6
     assert [ours.size(i) for i in range(6)] == [2] * 6          # fixed B1
-    assert theirs.size(0) == 6                                   # the reference bug
+    assert size0 == 6                                            # the reference bug
     GlobalSettings().reference_compat = True
     assert ours.size(0) == 6
     GlobalSettings().reference_compat = False
@@ -87,14 +93,18 @@ def test_sparse_and_networkx_topologies():
 
 
 def test_mixing_matches_reference(ref):
-    import gossipy.core as rc
     A = _ring(6); A[1, 3] = A[3, 1] = 1
-    ours, theirs = StaticP2PNetwork(6, A), rc.StaticP2PNetwork(6, A)
+
+    def theirs(rg):
+        net = rg.core.StaticP2PNetwork(6, A)
+        return [(np.asarray(rg.core.UniformMixing(net)[i]), np.asarray(rg.core.MetropolisHastingsMixing(net)[i]))
+                for i in range(6)]
+    weights = ref(theirs)
+    ours = StaticP2PNetwork(6, A)
     GlobalSettings().reference_compat = True      # node-0 degree quirk (B1) leaks into MH weights
     for i in range(6):
-        np.testing.assert_allclose(UniformMixing(ours)[i], rc.UniformMixing(theirs)[i])
-        np.testing.assert_allclose(MetropolisHastingsMixing(ours)[i],
-                                   rc.MetropolisHastingsMixing(theirs)[i])
+        np.testing.assert_allclose(UniformMixing(ours)[i], weights[i][0])
+        np.testing.assert_allclose(MetropolisHastingsMixing(ours)[i], weights[i][1])
     GlobalSettings().reference_compat = False
     assert len(UniformMixing(ours)[0]) == 3       # fixed: deg(0)+1, not num_nodes+1
     w = MetropolisHastingsMixing(ours, normalized=True)[1]

@@ -114,15 +114,18 @@ def test_recsys_and_loaders_offline():
 def test_assignment_strategies_reproduce_the_reference_splits_in_compat_mode(ref, name, kw, n, seed):
     """``reference_compat``: same seed -> the reference's index sets, element for element (and the same side effect
     on the global streams); the default draws from a private generator instead."""
-    import gossipy.data as RD
     import gossipy_b200 as g
     import gossipy_b200.data as OD
     y = torch.randint(0, 10, (1000,), generator=torch.Generator().manual_seed(0))
     g.GlobalSettings().reference_compat = True
     ours = getattr(OD.AssignmentHandler(seed), name)(y, n, **kw)
     probe_o = (float(np.random.rand()), float(torch.rand(1)))
-    theirs = getattr(RD.AssignmentHandler(seed), name)(y, n, **kw)
-    probe_r = (float(np.random.rand()), float(torch.rand(1)))
+
+    def theirs(rg):
+        split = getattr(rg.data.AssignmentHandler(seed), name)(y, n, **kw)
+        return [np.asarray(a) for a in split], (float(np.random.rand()), float(torch.rand(1)))
+    theirs, probe_r = ref(theirs)
+    probe_r = tuple(probe_r)
     assert len(ours) == len(theirs) == n
     for a, b in zip(ours, theirs):
         assert np.array_equal(np.asarray(a), np.asarray(b))
@@ -133,24 +136,41 @@ def test_assignment_strategies_reproduce_the_reference_splits_in_compat_mode(ref
 
 
 def test_train_test_split_and_auto_assignment_reproduce_the_reference_in_compat_mode(ref):
-    import gossipy.data as RD
-    import gossipy.data.handler as RH
     import gossipy_b200 as g
     import gossipy_b200.data as OD
     import gossipy_b200.data.handler as OH
     gen = torch.Generator().manual_seed(0)
     X = torch.randn(200, 5, generator=gen)
     y = torch.randint(0, 3, (200,), generator=gen)
+    splits = ((.2, 42), (.3, 7))
+
+    def rows(Xs):        # the rows of X (all distinct) that a split holds, in its order
+        pos = (torch.as_tensor(Xs)[:, None, :] == X[None]).all(-1).nonzero()
+        assert pos[:, 0].tolist() == list(range(len(Xs)))
+        return pos[:, 1]
+
+    def theirs(rg):
+        import gossipy.data.handler as RH
+        out = []
+        for ts, seed in splits:
+            b = RH.ClassificationDataHandler(X, y, test_size=ts, seed=seed)
+            out.append((rows(b.Xtr), b.ytr, rows(b.Xte), b.yte))
+        b = RH.ClassificationDataHandler(X.numpy(), y.numpy(), test_size=.25, seed=3)
+        out.append((rows(b.Xtr), b.yte))
+        b = rg.data.DataDispatcher(RH.ClassificationDataHandler(X, y, X[:40], y[:40]), n=7, eval_on_user=True,
+                                   auto_assign=True)
+        out.append(([np.asarray(p) for p in b.tr_assignments], [np.asarray(p) for p in b.te_assignments]))
+        return out
+    want = ref(theirs)
     g.GlobalSettings().reference_compat = True
-    for ts, seed in ((.2, 42), (.3, 7)):
+    for (ts, seed), (tr, ytr, te, yte) in zip(splits, want):
         a = OH.ClassificationDataHandler(X, y, test_size=ts, seed=seed)
-        b = RH.ClassificationDataHandler(X, y, test_size=ts, seed=seed)
-        for p, q in ((a.Xtr, b.Xtr), (a.ytr, b.ytr), (a.Xte, b.Xte), (a.yte, b.yte)):
+        for p, q in ((a.Xtr, X[tr]), (a.ytr, ytr), (a.Xte, X[te]), (a.yte, yte)):
             assert torch.equal(p, q)
     a = OH.ClassificationDataHandler(X.numpy(), y.numpy(), test_size=.25, seed=3)
-    b = RH.ClassificationDataHandler(X.numpy(), y.numpy(), test_size=.25, seed=3)
-    assert np.array_equal(a.Xtr, b.Xtr) and np.array_equal(a.yte, b.yte)
+    assert np.array_equal(a.Xtr, X.numpy()[want[2][0].numpy()]) and np.array_equal(a.yte, want[2][1])
     a = OD.DataDispatcher(OH.ClassificationDataHandler(X, y, X[:40], y[:40]), n=7, eval_on_user=True, auto_assign=True)
-    b = RD.DataDispatcher(RH.ClassificationDataHandler(X, y, X[:40], y[:40]), n=7, eval_on_user=True, auto_assign=True)
-    for p, q in list(zip(a.tr_assignments, b.tr_assignments)) + list(zip(a.te_assignments, b.te_assignments)):
-        assert np.array_equal(np.asarray(p), np.asarray(q))
+    tr, te = want[3]
+    assert len(a.tr_assignments) == len(tr) and len(a.te_assignments) == len(te)
+    for p, q in list(zip(a.tr_assignments, tr)) + list(zip(a.te_assignments, te)):
+        assert np.array_equal(np.asarray(p), q)

@@ -10,18 +10,23 @@ from gossipy_b200 import flow_control as fc
                                         ("GeneralizedTokenAccount", (8, 3)),
                                         ("RandomizedTokenAccount", (20, 10))])
 def test_tables_match_reference(ref, name, args):
-    import gossipy.flow_control as rfc
-    ours, theirs = getattr(fc, name)(*args), getattr(rfc, name)(*args)
-    for a in range(0, 45):
-        ours.n_tokens = theirs.n_tokens = a
-        assert ours.proactive() == pytest.approx(theirs.proactive())
-        for u in (0, 1, 2):
-            if name == "RandomizedTokenAccount":
-                np.random.seed(a * 7 + u); r1 = ours.reactive(u)
-                np.random.seed(a * 7 + u); r2 = theirs.reactive(u)
-                assert r1 == r2
-            else:
-                assert ours.reactive(u) == theirs.reactive(u)
+    def table(module):
+        acc = getattr(module, name)(*args)
+        rows = []
+        for a in range(0, 45):
+            acc.n_tokens = a
+            row = [acc.proactive()]
+            for u in (0, 1, 2):
+                if name == "RandomizedTokenAccount":
+                    np.random.seed(a * 7 + u)
+                row.append(acc.reactive(u))
+            rows.append(row)
+        return rows
+    ours, theirs = table(fc), ref(lambda rg: table(rg.flow_control))
+    assert len(ours) == len(theirs) == 45
+    for a, (o, t) in enumerate(zip(ours, theirs)):
+        assert o[0] == pytest.approx(t[0]), a
+        assert o[1:] == t[1:], a
 
 
 def test_add_sub_and_proactive_account():

@@ -22,51 +22,73 @@ def _data(n=96, d=12, c=3, seed=0):
     return X, (X @ torch.randn(d, c, generator=gen)).argmax(1)
 
 
-def _pair(ref, cls_name, net_fn, **kw):
-    """Our handler and the reference's, with identical initial weights."""
-    import gossipy.model.handler as RH
-    import gossipy.model.nn as RN
-    ours_net = net_fn(g.model.nn)
-    theirs_net = net_fn(RN)
-    theirs_net.load_state_dict(ours_net.state_dict())
+def _common(kw):
     common = dict(optimizer=torch.optim.SGD, optimizer_params={"lr": .1, "weight_decay": .01},
                   criterion=CE, batch_size=0, local_epochs=1)
     common.update(kw)
-    ours = getattr(H, cls_name)(net=ours_net, **common)
-    okw = dict(common)
+    return common
+
+
+def _ours(cls_name, net_fn, **kw):
+    return getattr(H, cls_name)(net=net_fn(g.model.nn), **_common(kw))
+
+
+def _theirs(cls_name, net_fn, **kw):
+    """The original gossipy's handler with the same arguments."""
+    import gossipy.model.handler as RH
+    import gossipy.model.nn as RN
+    okw = _common(kw)
     if "create_model_mode" in okw:
         okw["create_model_mode"] = getattr(RH.CreateModelMode, okw["create_model_mode"].name)
-    theirs = getattr(RH, cls_name)(net=theirs_net, **okw)
-    return ours, theirs
+    return getattr(RH, cls_name)(net=net_fn(RN), **okw)
 
 
 def _flat(module):
     return torch.cat([p.detach().reshape(-1) for p in module.parameters()])
 
 
-def _set_random(ours, theirs, seed):
+def _randn_params(module, seed):
     gen = torch.Generator().manual_seed(seed)
-    for p in theirs.model.parameters():
-        p.data = torch.randn(p.shape, generator=gen)
-    ours.model.load_state_dict(theirs.model.state_dict())
+    return [torch.randn(p.shape, generator=gen) for p in module.parameters()]
+
+
+def _set_random(ours, seed):
+    names = [n for n, _ in ours.model.named_parameters()]
+    ours.model.load_state_dict(dict(zip(names, _randn_params(ours.model, seed))))
     ours.model = ours.model  # re-gather into the row
+
+
+def _set_random_theirs(theirs, seed):
+    for p, v in zip(list(theirs.model.parameters()), _randn_params(theirs.model, seed)):
+        p.data = v
 
 
 def test_fullbatch_update_and_uniform_merge_match_reference(ref):
     X, y = _data()
     mk = lambda ns: ns.TorchMLP(12, 3, (8,))
-    a, ra = _pair(ref, "TorchModelHandler", mk)
-    b, rb = _pair(ref, "TorchModelHandler", mk)
-    _set_random(a, ra, 1); _set_random(b, rb, 2)
-    for h in (a, ra, b, rb):
+
+    def theirs(rg):
+        ra, rb = _theirs("TorchModelHandler", mk), _theirs("TorchModelHandler", mk)
+        _set_random_theirs(ra, 1); _set_random_theirs(rb, 2)
+        for h in (ra, rb):
+            h._update((X, y))
+        out = [ra.n_updates, _flat(ra.model)]
+        ra._merge(rb)
+        out.append(_flat(ra.model))
+        ra._merge([rb, rb])
+        return out + [_flat(ra.model), ra.evaluate((X, y))]
+    r_updates, r_upd, r_merge, r_merge2, rev = ref(theirs)
+    a, b = _ours("TorchModelHandler", mk), _ours("TorchModelHandler", mk)
+    _set_random(a, 1); _set_random(b, 2)
+    for h in (a, b):
         h._update((X, y))
-    assert a.n_updates == ra.n_updates == 1
-    torch.testing.assert_close(_flat(a.model), _flat(ra.model), rtol=1e-5, atol=1e-6)
-    a._merge(b); ra._merge(rb)
-    torch.testing.assert_close(_flat(a.model), _flat(ra.model), rtol=1e-5, atol=1e-6)
-    a._merge([b, b]); ra._merge([rb, rb])
-    torch.testing.assert_close(_flat(a.model), _flat(ra.model), rtol=1e-5, atol=1e-6)
-    ev, rev = a.evaluate((X, y)), ra.evaluate((X, y))
+    assert a.n_updates == r_updates == 1
+    torch.testing.assert_close(_flat(a.model), r_upd, rtol=1e-5, atol=1e-6)
+    a._merge(b)
+    torch.testing.assert_close(_flat(a.model), r_merge, rtol=1e-5, atol=1e-6)
+    a._merge([b, b])
+    torch.testing.assert_close(_flat(a.model), r_merge2, rtol=1e-5, atol=1e-6)
+    ev = a.evaluate((X, y))
     for k in rev:
         assert ev[k] == pytest.approx(float(rev[k]), abs=1e-6), k
 
@@ -119,60 +141,95 @@ def test_flat_optimizers_match_torch(opt, params):
 def test_modes_match_reference(ref):
     X, y = _data()
     mk = lambda ns: ns.LogisticRegression(12, 3)
-    for mode in (M.UPDATE, M.MERGE_UPDATE, M.UPDATE_MERGE, M.PASS):
-        a, ra = _pair(ref, "TorchModelHandler", mk, create_model_mode=mode)
-        b, rb = _pair(ref, "TorchModelHandler", mk, create_model_mode=mode)
-        _set_random(a, ra, 3); _set_random(b, rb, 4)
-        b.n_updates = rb.n_updates = 5
-        a(b.copy(), (X, y)); ra(rb.copy(), (X, y))
-        assert a.n_updates == ra.n_updates, mode
-        torch.testing.assert_close(_flat(a.model), _flat(ra.model), rtol=1e-5, atol=1e-6, msg=str(mode))
+    modes = (M.UPDATE, M.MERGE_UPDATE, M.UPDATE_MERGE, M.PASS)
+
+    def theirs(rg):
+        out = []
+        for mode in modes:
+            ra, rb = _theirs("TorchModelHandler", mk, create_model_mode=mode), \
+                _theirs("TorchModelHandler", mk, create_model_mode=mode)
+            _set_random_theirs(ra, 3); _set_random_theirs(rb, 4)
+            rb.n_updates = 5
+            ra(rb.copy(), (X, y))
+            out.append((ra.n_updates, _flat(ra.model)))
+        return out
+    for mode, (r_updates, r_flat) in zip(modes, ref(theirs)):
+        a, b = _ours("TorchModelHandler", mk, create_model_mode=mode), _ours("TorchModelHandler", mk, create_model_mode=mode)
+        _set_random(a, 3); _set_random(b, 4)
+        b.n_updates = 5
+        a(b.copy(), (X, y))
+        assert a.n_updates == r_updates, mode
+        torch.testing.assert_close(_flat(a.model), r_flat, rtol=1e-5, atol=1e-6, msg=str(mode))
 
 
 def test_limited_merge_branches(ref):
     mk = lambda ns: ns.LogisticRegression(12, 3)
-    for na, nb in ((10, 2), (2, 10), (4, 5), (0, 0)):
-        a, ra = _pair(ref, "LimitedMergeTMH", mk, age_diff_threshold=1)
-        b, rb = _pair(ref, "LimitedMergeTMH", mk, age_diff_threshold=1)
-        _set_random(a, ra, 5); _set_random(b, rb, 6)
-        a.n_updates = ra.n_updates = na
-        b.n_updates = rb.n_updates = nb
-        a._merge(b)
-        if (na, nb) != (0, 0):   # the reference divides by zero for two fresh models
+    ages = ((10, 2), (2, 10), (4, 5))   # the reference divides by zero for two fresh models: (0, 0) is ours only
+
+    def theirs(rg):
+        out = []
+        for na, nb in ages:
+            ra, rb = _theirs("LimitedMergeTMH", mk, age_diff_threshold=1), _theirs("LimitedMergeTMH", mk, age_diff_threshold=1)
+            _set_random_theirs(ra, 5); _set_random_theirs(rb, 6)
+            ra.n_updates, rb.n_updates = na, nb
             ra._merge(rb)
-            torch.testing.assert_close(_flat(a.model), _flat(ra.model), rtol=1e-5, atol=1e-6)
-            assert a.n_updates == ra.n_updates
+            out.append((_flat(ra.model), ra.n_updates))
+        return out
+    want = ref(theirs)
+    for i, (na, nb) in enumerate(ages + ((0, 0),)):
+        a, b = _ours("LimitedMergeTMH", mk, age_diff_threshold=1), _ours("LimitedMergeTMH", mk, age_diff_threshold=1)
+        _set_random(a, 5); _set_random(b, 6)
+        a.n_updates, b.n_updates = na, nb
+        a._merge(b)
+        if i < len(ages):
+            torch.testing.assert_close(_flat(a.model), want[i][0], rtol=1e-5, atol=1e-6)
+            assert a.n_updates == want[i][1]
         else:
             assert torch.isfinite(a.row).all()
 
 
 def test_weighted_kway_merge(ref):
     mk = lambda ns: ns.LogisticRegression(12, 3)
-    hs = [_pair(ref, "WeightedTMH", mk) for _ in range(4)]
-    for i, (o, r) in enumerate(hs):
-        _set_random(o, r, 10 + i)
     w = np.array([.4, .3, .2, .1])
-    hs[0][0]._merge([h[0] for h in hs[1:]], w)
-    hs[0][1]._merge([h[1] for h in hs[1:]], w)
-    torch.testing.assert_close(_flat(hs[0][0].model), _flat(hs[0][1].model), rtol=1e-5, atol=1e-6)
+
+    def theirs(rg):
+        hs = [_theirs("WeightedTMH", mk) for _ in range(4)]
+        for i, h in enumerate(hs):
+            _set_random_theirs(h, 10 + i)
+        hs[0]._merge(hs[1:], w)
+        return _flat(hs[0].model)
+    want = ref(theirs)
+    hs = [_ours("WeightedTMH", mk) for _ in range(4)]
+    for i, h in enumerate(hs):
+        _set_random(h, 10 + i)
+    hs[0]._merge(hs[1:], w)
+    torch.testing.assert_close(_flat(hs[0].model), want, rtol=1e-5, atol=1e-6)
 
 
 def test_partition_index_sets_and_merge_match_reference(ref):
-    import gossipy.model.sampling as RS
-    import gossipy.model.nn as RN
-    for net_o, net_r, parts in ((LogisticRegression(5, 2), RN.LogisticRegression(5, 2), 4),
-                                (TorchMLP(7, 3, (5,)), RN.TorchMLP(7, 3, (5,)), 3),
-                                (TorchMLP(7, 3, (5,)), RN.TorchMLP(7, 3, (5,)), 7)):
-        po, pr = TorchModelPartition(net_o, parts), RS.TorchModelPartition(net_r, parts)
-        assert po.n_parts == pr.n_parts
+    setups = ((lambda ns: ns.LogisticRegression(5, 2), 4), (lambda ns: ns.TorchMLP(7, 3, (5,)), 3),
+              (lambda ns: ns.TorchMLP(7, 3, (5,)), 7))
+
+    def theirs(rg):
+        import gossipy.model.nn as RN
+        import gossipy.model.sampling as RS
+        out = []
+        for mk, parts in setups:
+            pr = RS.TorchModelPartition(mk(RN), parts)
+            out.append((pr.n_parts, [[(ti, None if ids is None else [x.tolist() for x in ids])
+                                      for ti, ids in pr.partitions[p].items()] for p in range(pr.n_parts)]))
+        return out
+    for (mk, parts), (n_parts, partitions) in zip(setups, ref(theirs)):
+        po = TorchModelPartition(mk(g.model.nn), parts)
+        assert po.n_parts == n_parts
         flat_all = []
         for p in range(po.n_parts):
-            for ti, ids in pr.partitions[p].items():
+            for ti, ids in partitions[p]:
                 mine = po.partitions[p][ti]
                 if ids is None:
                     assert mine is None
                     continue
-                a = sorted(zip(*[x.tolist() for x in ids]))
+                a = sorted(zip(*ids))
                 b = sorted(zip(*[x.tolist() for x in mine]))
                 assert a == b, (p, ti)
             # segments cover exactly the flat index set
@@ -185,38 +242,52 @@ def test_partition_index_sets_and_merge_match_reference(ref):
 
 
 def test_partitioned_handler_matches_reference(ref):
-    import gossipy.model.sampling as RS
     X, y = _data()
     mk = lambda ns: ns.TorchMLP(12, 3, (6,))
-    import gossipy.model.nn as RN
-    a, ra = _pair(ref, "PartitionedTMH", mk, tm_partition=TorchModelPartition(mk(g.model.nn), 4))
-    b, rb = _pair(ref, "PartitionedTMH", mk, tm_partition=TorchModelPartition(mk(g.model.nn), 4))
-    for r_ in (ra, rb):
-        r_.tm_partition = RS.TorchModelPartition(mk(RN), 4)
-    _set_random(a, ra, 7); _set_random(b, rb, 8)
-    for h in (a, ra):
-        h._update((X, y)); h._update((X, y))
-    for h in (b, rb):
-        h._update((X, y))
-    assert a.n_updates.tolist() == ra.n_updates.tolist() == [2] * 4
-    torch.testing.assert_close(_flat(a.model), _flat(ra.model), rtol=1e-5, atol=1e-6)
-    a._merge(b, 2); ra._merge(rb, 2)
-    a._merge(b, 5); ra._merge(rb, 1)      # ours wraps the id modulo n_parts
-    torch.testing.assert_close(_flat(a.model), _flat(ra.model), rtol=1e-5, atol=1e-6)
-    assert a.n_updates.tolist() == ra.n_updates.tolist()
+
+    def theirs(rg):
+        import gossipy.model.nn as RN
+        import gossipy.model.sampling as RS
+        ra, rb = (_theirs("PartitionedTMH", mk, tm_partition=RS.TorchModelPartition(mk(RN), 4)) for _ in range(2))
+        _set_random_theirs(ra, 7); _set_random_theirs(rb, 8)
+        ra._update((X, y)); ra._update((X, y))
+        rb._update((X, y))
+        out = [ra.n_updates.tolist(), _flat(ra.model)]
+        ra._merge(rb, 2)
+        ra._merge(rb, 1)
+        return out + [_flat(ra.model), ra.n_updates.tolist()]
+    r_updates, r_upd, r_merge, r_updates2 = ref(theirs)
+    a = _ours("PartitionedTMH", mk, tm_partition=TorchModelPartition(mk(g.model.nn), 4))
+    b = _ours("PartitionedTMH", mk, tm_partition=TorchModelPartition(mk(g.model.nn), 4))
+    _set_random(a, 7); _set_random(b, 8)
+    a._update((X, y)); a._update((X, y))
+    b._update((X, y))
+    assert a.n_updates.tolist() == r_updates == [2] * 4
+    torch.testing.assert_close(_flat(a.model), r_upd, rtol=1e-5, atol=1e-6)
+    a._merge(b, 2)
+    a._merge(b, 5)      # ours wraps the id modulo n_parts (the reference is given 1)
+    torch.testing.assert_close(_flat(a.model), r_merge, rtol=1e-5, atol=1e-6)
+    assert a.n_updates.tolist() == r_updates2
     assert a.caching(0).key[1] == str(a.n_updates)
     CACHE.clear()
 
 
 def test_sampled_merge_matches_reference(ref):
-    import gossipy.model.sampling as RS
     mk = lambda ns: ns.TorchMLP(12, 3, (6,))
-    a, ra = _pair(ref, "SamplingTMH", mk, sample_size=.3)
-    b, rb = _pair(ref, "SamplingTMH", mk, sample_size=.3)
-    _set_random(a, ra, 9); _set_random(b, rb, 10)
-    sample = RS.TorchModelSampling.sample(.3, ra.model)
-    a._merge(b, sample); ra._merge(rb, sample)
-    torch.testing.assert_close(_flat(a.model), _flat(ra.model), rtol=1e-6, atol=1e-7)
+
+    def theirs(rg):
+        import gossipy.model.sampling as RS
+        ra, rb = _theirs("SamplingTMH", mk, sample_size=.3), _theirs("SamplingTMH", mk, sample_size=.3)
+        _set_random_theirs(ra, 9); _set_random_theirs(rb, 10)
+        sample = RS.TorchModelSampling.sample(.3, ra.model)
+        ra._merge(rb, sample)
+        return sample, _flat(ra.model)
+    sample, want = ref(theirs)
+    sample = {k: None if v is None else tuple(v) for k, v in sample.items()}
+    a, b = _ours("SamplingTMH", mk, sample_size=.3), _ours("SamplingTMH", mk, sample_size=.3)
+    _set_random(a, 9); _set_random(b, 10)
+    a._merge(b, sample)
+    torch.testing.assert_close(_flat(a.model), want, rtol=1e-6, atol=1e-7)
     flat = a.draw_sample()
     assert flat.numel() == round(.3 * a.get_size()) and int(flat.max()) < a.get_size()
     d = TorchModelSampling.sample(.5, a.model)
@@ -224,61 +295,87 @@ def test_sampled_merge_matches_reference(ref):
 
 
 def test_adaline_and_pegasos_match_reference(ref):
-    import gossipy.model.handler as RH
-    import gossipy.model.nn as RN
     gen = torch.Generator().manual_seed(0)
     X = torch.randn(40, 9, generator=gen)
     y = torch.sign(X @ torch.randn(9, generator=gen))
-    for name, lr in (("AdaLineHandler", .01), ("PegasosHandler", .01)):
+    learners = (("AdaLineHandler", .01), ("PegasosHandler", .01))
+
+    def theirs(rg):
+        import gossipy.model.handler as RH
+        import gossipy.model.nn as RN
+        out = []
+        for name, lr in learners:
+            r = getattr(RH, name)(RN.AdaLine(9), lr)
+            r.init()
+            r._update((X, y)); r._update((X[:7], y[:7]))
+            res = [r.n_updates, r.model.model.detach().clone()]
+            r2 = copy.deepcopy(r); r2._update((X[:3], y[:3]))
+            r._merge(r2)
+            out.append(res + [r.model.model.detach().clone(), r.evaluate((X, y))])
+        return out
+    for (name, lr), (r_updates, r_upd, r_merge, er) in zip(learners, ref(theirs)):
         o = getattr(H, name)(AdaLine(9), lr)
-        r = getattr(RH, name)(RN.AdaLine(9), lr)
-        o.init(); r.init()
-        o._update((X, y)); r._update((X, y))
-        o._update((X[:7], y[:7])); r._update((X[:7], y[:7]))
-        assert o.n_updates == r.n_updates == 47
-        torch.testing.assert_close(o.model.model.detach(), r.model.model.detach(), rtol=1e-4, atol=1e-5)
+        o.init()
+        o._update((X, y)); o._update((X[:7], y[:7]))
+        assert o.n_updates == r_updates == 47
+        torch.testing.assert_close(o.model.model.detach(), r_upd, rtol=1e-4, atol=1e-5)
         o2 = o.copy(); o2._update((X[:3], y[:3]))
-        r2 = copy.deepcopy(r); r2._update((X[:3], y[:3]))
-        o._merge(o2); r._merge(r2)
-        torch.testing.assert_close(o.model.model.detach(), r.model.model.detach(), rtol=1e-4, atol=1e-5)
-        eo, er = o.evaluate((X, y)), r.evaluate((X, y))
+        o._merge(o2)
+        torch.testing.assert_close(o.model.model.detach(), r_merge, rtol=1e-4, atol=1e-5)
+        eo = o.evaluate((X, y))
         for k in er:
             assert eo[k] == pytest.approx(float(er[k]), abs=1e-6)
 
 
 def test_kmeans_and_mf_match_reference(ref):
-    import gossipy.model.handler as RH
     gen = torch.Generator().manual_seed(0)
     X = torch.randn(60, 5, generator=gen); yl = (X[:, 0] > 0).long()
-    o, r = H.KMeansHandler(3, 5, alpha=.2), RH.KMeansHandler(3, 5, alpha=.2)
-    o.init(); r.init()
-    o.model = r.model.clone()
-    o._update((X[:1], None)); r._update((X[:1], None))
-    o._update((X[1:9], None)); r._update((X[1:9], None))
-    torch.testing.assert_close(o.model, r.model)
-    assert o.evaluate((X, yl))["nmi"] == pytest.approx(r.evaluate((X, yl))["nmi"])
+    ratings = np.array([(1, 4.), (3, 2.), (0, 5.), (1, 1.)])
+
+    def theirs(rg):
+        import gossipy.model.handler as RH
+        r = RH.KMeansHandler(3, 5, alpha=.2)
+        r.init()
+        init = r.model.clone()
+        r._update((X[:1], None)); r._update((X[1:9], None))
+        km = [init, r.model.clone(), r.evaluate((X, yl))["nmi"]]
+        mr = RH.MFModelHandler(4, 6)
+        mr.init()
+        mf = [copy.deepcopy(mr.model)]
+        mr._update(ratings)
+        mf += [mr.model[1][0].copy(), mr.model[0][0].copy(), mr.n_updates]
+        r2 = copy.deepcopy(mr)
+        r2._update(ratings[:2])
+        mr._merge(r2)
+        return km + mf + [mr.model[1][0].copy(), mr.model[1][1].copy(), mr.evaluate(ratings)["rmse"], mr.get_size()]
+    (k_init, k_upd, nmi, mf_init, mf_y, mf_x, mf_updates,
+     mf_y_merged, mf_c_merged, rmse, mf_size) = ref(theirs)
+    o = H.KMeansHandler(3, 5, alpha=.2)
+    o.init()
+    o.model = k_init.clone()
+    o._update((X[:1], None)); o._update((X[1:9], None))
+    torch.testing.assert_close(o.model, k_upd)
+    assert o.evaluate((X, yl))["nmi"] == pytest.approx(nmi)
     o2 = o.copy(); o2.model = o.model.flip(0)
     hung = H.KMeansHandler(3, 5, matching="hungarian"); hung.init(); hung.model = o.model.clone()
     hung._merge(o2)                       # optimal matching undoes the flip (B16 fixed)
     torch.testing.assert_close(hung.model, o.model)
     # matrix factorisation
-    ratings = np.array([(1, 4.), (3, 2.), (0, 5.), (1, 1.)])
-    mo, mr = H.MFModelHandler(4, 6), RH.MFModelHandler(4, 6)
-    mo.init(); mr.init()
-    mo.model = copy.deepcopy(mr.model)
-    mo._update(ratings); mr._update(ratings)
-    np.testing.assert_allclose(mo.model[1][0], mr.model[1][0], rtol=1e-5, atol=1e-6)
-    np.testing.assert_allclose(mo.model[0][0], mr.model[0][0], rtol=1e-5, atol=1e-6)
-    assert mo.n_updates == mr.n_updates == 5
-    m2, r2 = mo.copy(), copy.deepcopy(mr)
-    m2._update(ratings[:2]); r2._update(ratings[:2])
-    mo._merge(m2); mr._merge(r2)
-    np.testing.assert_allclose(mo.model[1][0], mr.model[1][0], rtol=1e-5, atol=1e-6)
-    np.testing.assert_allclose(mo.model[1][1], mr.model[1][1], rtol=1e-5, atol=1e-6)
-    assert mo.evaluate(ratings)["rmse"] == pytest.approx(mr.evaluate(ratings)["rmse"], rel=1e-5)
-    assert mo.get_size() == mr.get_size() == 4 * 7
-
-
+    mo = H.MFModelHandler(4, 6)
+    mo.init()
+    (Xu, b), (Y, c) = mf_init
+    mo.model = ((Xu, b), (Y, c))
+    mo._update(ratings)
+    np.testing.assert_allclose(mo.model[1][0], mf_y, rtol=1e-5, atol=1e-6)
+    np.testing.assert_allclose(mo.model[0][0], mf_x, rtol=1e-5, atol=1e-6)
+    assert mo.n_updates == mf_updates == 5
+    m2 = mo.copy()
+    m2._update(ratings[:2])
+    mo._merge(m2)
+    np.testing.assert_allclose(mo.model[1][0], mf_y_merged, rtol=1e-5, atol=1e-6)
+    np.testing.assert_allclose(mo.model[1][1], mf_c_merged, rtol=1e-5, atol=1e-6)
+    assert mo.evaluate(ratings)["rmse"] == pytest.approx(rmse, rel=1e-5)
+    assert mo.get_size() == mf_size == 4 * 7
 def test_batchnorm_model_merges():
     """B12: the reference crashes merging BN models; here float buffers average, counters max."""
     gen = torch.Generator().manual_seed(0)

@@ -85,17 +85,43 @@ def _logreg_proto(mode="MERGE_UPDATE", cls="TorchModelHandler", **extra):
     return fn
 
 
+class _Recorded:
+    """What the comparisons read of a finished run of the original gossipy: message counters, evaluations, node ages."""
+
+    def __init__(self, d):
+        self._sent_messages, self._failed_messages, self._total_size = d["sent"], d["failed"], d["size"]
+        self._eval = {False: [tuple(e) for e in d["global"]], True: [tuple(e) for e in d["local"]]}
+        self.n_updates = d["n_updates"]
+
+    def get_evaluation(self, local=False):
+        return self._eval[local]
+
+
+def _summary(rep, sim):
+    def ev(local):
+        return [(t, {k: float(v) for k, v in e.items()}) for t, e in rep.get_evaluation(local)]
+    return {"sent": rep._sent_messages, "failed": rep._failed_messages, "size": rep._total_size,
+            "global": ev(False), "local": ev(True),
+            "n_updates": [np.asarray(sim.nodes[i].model_handler.n_updates).tolist() for i in sorted(sim.nodes)]}
+
+
+def _reference_run(ref, run):
+    """``run(ns)`` -> (report, simulator) on the original gossipy, as recorded."""
+    return _Recorded(ref(lambda rg: _summary(*run(_ns(rg)))))
+
+
+def _run_one(ns, rounds=4, **kw):
+    sim, rep, _ = _build(ns, **kw)
+    random.seed(11); np.random.seed(11); torch.manual_seed(11)
+    sim.init_nodes(seed=42)
+    random.seed(12); np.random.seed(12)
+    sim.start(n_rounds=rounds)
+    rep.sim = sim
+    return rep, sim
+
+
 def _run_both(ref, rounds=4, **kw):
-    out = []
-    for ns in (_ns(), _ns(ref)):
-        sim, rep, _ = _build(ns, **kw)
-        random.seed(11); np.random.seed(11); torch.manual_seed(11)
-        sim.init_nodes(seed=42)
-        random.seed(12); np.random.seed(12)
-        sim.start(n_rounds=rounds)
-        rep.sim = sim
-        out.append(rep)
-    return out
+    return _run_one(_ns(), rounds, **kw)[0], _reference_run(ref, lambda ns: _run_one(ns, rounds, **kw))
 
 
 @pytest.mark.parametrize("protocol", ["PUSH", "PULL", "PUSH_PULL"])
@@ -184,8 +210,7 @@ def test_all2all_uniform_clique_is_global_average(ref):
         torch.manual_seed(0)
         return ns["handler"].WeightedTMH(net=ns["nn"].LogisticRegression(10, 2), optimizer=torch.optim.SGD,
                                          optimizer_params={"lr": .5}, criterion=CE, batch_size=0)
-    reps = []
-    for ns in (_ns(), _ns(ref)):
+    def run(ns):
         sim, rep, net = _build(ns, n_nodes=6, proto_fn=proto, node_cls="All2AllGossipNode",
                                sim_cls="All2AllGossipSimulator")
         random.seed(11); np.random.seed(11); torch.manual_seed(11)
@@ -193,8 +218,8 @@ def test_all2all_uniform_clique_is_global_average(ref):
         random.seed(12); np.random.seed(12)
         sim.start(ns["core"].UniformMixing(net), n_rounds=4)
         rep.sim = sim
-        reps.append(rep)
-    ours, theirs = reps
+        return rep, sim
+    ours, theirs = run(_ns())[0], _reference_run(ref, run)
     assert (ours._sent_messages, ours._total_size) == (theirs._sent_messages, theirs._total_size)
     a, b = ours.get_evaluation(False)[-1][1], theirs.get_evaluation(False)[-1][1]
     # node 0 uses deg+1 weights here but num_nodes+1 in the reference (B1): allow a small gap
@@ -320,7 +345,7 @@ def test_random_setups_match_reference(ref):
         if not (mode == "MERGE_UPDATE" or one_per_round):
             return
         assert [int(ours.sim.nodes[i].model_handler.n_updates) for i in range(n_nodes)] == \
-            [int(theirs.sim.nodes[i].model_handler.n_updates) for i in range(n_nodes)]
+            [int(theirs.n_updates[i]) for i in range(n_nodes)]
         for (_, a), (_, b) in list(zip(eo, er)) + list(zip(lo, lr_)):
             for k in b:
                 assert a[k] == pytest.approx(float(b[k]), abs=2.5 / (80 * n_nodes)), (k, protocol, mode)   # <= 2 borderline samples
@@ -356,8 +381,7 @@ def test_sampled_and_partitioned_nodes_match_reference_exactly(ref, node_cls, pr
 
 
 def _run_both_built(ref, build, rounds=3):
-    out = []
-    for ns in (_ns(), _ns(ref)):
+    def run(ns):
         random.seed(5); np.random.seed(5); torch.manual_seed(5)
         sim, rep = build(ns)
         if hasattr(sim, "progress"):
@@ -367,8 +391,8 @@ def _run_both_built(ref, build, rounds=3):
         random.seed(12); np.random.seed(12)
         sim.start(n_rounds=rounds)
         rep.sim = sim
-        out.append(rep)
-    return out
+        return rep, sim
+    return run(_ns())[0], _reference_run(ref, run)
 
 
 def _assert_same_run(ours, theirs, curves=True, tol=1e-6):
@@ -503,8 +527,7 @@ def test_all2all_matches_reference_exactly_in_compat_mode(ref, mixing, topo_kind
         sim.add_receiver(rep)
         sim._W = getattr(ns["core"], mixing)(net)
         return sim, rep
-    out = []
-    for ns in (_ns(), _ns(ref)):
+    def run(ns):
         random.seed(5); np.random.seed(5); torch.manual_seed(5)
         sim, rep = build(ns)
         if hasattr(sim, "progress"):
@@ -513,8 +536,8 @@ def test_all2all_matches_reference_exactly_in_compat_mode(ref, mixing, topo_kind
         sim.init_nodes(seed=42)
         random.seed(12); np.random.seed(12)
         sim.start(sim._W, n_rounds=3)
-        out.append(rep)
-    _assert_same_run(out[0], out[1])
+        return rep, sim
+    _assert_same_run(run(_ns())[0], _reference_run(ref, run))
 
 
 _ACCOUNTS = {"proactive": lambda ns: ns["fc"].PurelyProactiveTokenAccount(),
@@ -593,7 +616,7 @@ def test_limited_merge_matches_reference_exactly(ref, L, protocol, faults):
                              protocol=protocol, sim_kw=kw, sync=False)
     _assert_same_run(ours, theirs)
     assert [int(ours.sim.nodes[i].model_handler.n_updates) for i in range(8)] == \
-        [int(theirs.sim.nodes[i].model_handler.n_updates) for i in range(8)]
+        [int(theirs.n_updates[i]) for i in range(8)]
 
 
 @pytest.mark.parametrize("net_kind", ["logreg", "mlp"])
@@ -620,7 +643,7 @@ def test_minibatch_training_matches_reference_exactly(ref, net_kind, bs, epochs,
     ours, theirs = _run_both(ref, rounds=3, n_nodes=4, proto_fn=proto, protocol="PUSH_PULL", sim_kw=kw)
     _assert_same_run(ours, theirs, tol=1e-9)
     assert [int(ours.sim.nodes[i].model_handler.n_updates) for i in range(4)] == \
-        [int(theirs.sim.nodes[i].model_handler.n_updates) for i in range(4)]
+        [int(theirs.n_updates[i]) for i in range(4)]
 
 
 def test_whole_script_pipeline_matches_reference_in_compat_mode(ref):
@@ -632,8 +655,7 @@ def test_whole_script_pipeline_matches_reference_in_compat_mode(ref):
     gen = torch.Generator().manual_seed(3)
     X = torch.randn(600, 12, generator=gen)
     y = (X @ torch.randn(12, 2, generator=gen)).argmax(1)
-    out = []
-    for ns, root in ((_ns(), g), (_ns(ref), ref)):
+    def run(ns, root):
         root.set_seed(98765)
         dh = ns["data_handler"].ClassificationDataHandler(X, y, test_size=.1)
         disp = ns["data"].DataDispatcher(dh, n=20, eval_on_user=False, auto_assign=True)
@@ -657,5 +679,6 @@ def test_whole_script_pipeline_matches_reference_in_compat_mode(ref):
         sim.add_receiver(rep)
         sim.init_nodes(seed=42)
         sim.start(n_rounds=6)
-        out.append(rep)
-    _assert_same_run(out[0], out[1], tol=1e-9)
+        return rep, sim
+    ours = run(_ns(), g)[0]
+    _assert_same_run(ours, _Recorded(ref(lambda rg: _summary(*run(_ns(rg), rg)))), tol=1e-9)
