@@ -7,7 +7,9 @@ of :mod:`gossipy_b200.data.synthetic` (``load_*`` fall back to them automaticall
 
 Environment: ``GOSSIPY_ROUNDS`` (override the number of rounds), ``GOSSIPY_NODES`` (cap the number
 of nodes), ``GOSSIPY_ENGINE=native|python`` (round-loop control plane), ``GOSSIPY_EXECUTOR=native``
-(with the native engine: enqueue eligible simulations from the C++ executor), ``GOSSIPY_DEVICE``,
+(with the native engine: enqueue eligible simulations from the C++ executor), ``GOSSIPY_BATCHED=auto|0|1``
+(with the native engine: run bankable set-ups many nodes per launch -- ``auto``: on a GPU or from 512 nodes),
+``GOSSIPY_DEVICE``,
 ``GOSSIPY_COMPAT=1`` (``reference_compat``: reproduce the reference's numbers, Python engine).
 Multi-GPU: launch with ``python -m torch.distributed.run --nproc-per-node N examples/<script>.py``.
 """
@@ -55,6 +57,7 @@ def configure(sim):
     sim.engine = os.environ.get("GOSSIPY_ENGINE", "python")
     sim.native_executor = os.environ.get("GOSSIPY_EXECUTOR", "python") == "native"
     sim.progress = os.environ.get("GOSSIPY_PROGRESS", "0") == "1"
+    sim.batched = {"auto": "auto", "0": False, "1": True}[os.environ.get("GOSSIPY_BATCHED", "auto")]
     return sim
 
 

@@ -459,6 +459,76 @@ at::Tensor bank_scores(BANK_ARGS, at::Tensor nodes, at::Tensor Xte) {
     return out;
 }
 
+// ---- banks of k-means / matrix-factorisation models --------------------------------------------------------
+static FamilyBankView family_view(at::Tensor W, at::Tensor age, at::Tensor S, at::Tensor slot_age, at::Tensor data,
+                                  at::Tensor off, at::Tensor cnt, int64_t k, int64_t dim, int64_t mode, bool hungarian,
+                                  double alpha, double reg, double lr) {
+    TORCH_CHECK(W.is_cuda() && W.scalar_type() == at::kFloat && W.is_contiguous() && W.dim() == 2 && W.size(1) % 32 == 0);
+    TORCH_CHECK(S.is_cuda() && S.scalar_type() == at::kFloat && S.is_contiguous() && S.dim() == 2 && S.size(1) == W.size(1));
+    TORCH_CHECK(age.scalar_type() == at::kLong && slot_age.scalar_type() == at::kLong && off.scalar_type() == at::kLong &&
+                cnt.scalar_type() == at::kInt && data.scalar_type() == at::kFloat);
+    TORCH_CHECK(data.is_contiguous() && off.numel() == W.size(0) && cnt.numel() == W.size(0) &&
+                age.numel() == W.size(0) && slot_age.numel() == S.size(0));
+    FamilyBankView b{};
+    b.W = W.data_ptr<float>(); b.age = reinterpret_cast<long long*>(age.data_ptr<int64_t>());
+    b.S = S.data_ptr<float>(); b.slot_age = reinterpret_cast<long long*>(slot_age.data_ptr<int64_t>());
+    b.Dp = (int)W.size(1);
+    b.data = data.data_ptr<float>(); b.off = off.data_ptr<int64_t>(); b.cnt = cnt.data_ptr<int>();
+    b.k = (int)k; b.dim = (int)dim; b.mode = (int)mode; b.hungarian = hungarian ? 1 : 0;
+    b.alpha = (float)alpha; b.reg = (float)reg; b.lr = (float)lr;
+    return b;
+}
+#define FAMILY_ARGS at::Tensor W, at::Tensor age, at::Tensor S, at::Tensor slot_age, at::Tensor data, at::Tensor off, \
+                    at::Tensor cnt, int64_t k, int64_t dim, int64_t mode, bool hungarian, double alpha, double reg, double lr
+#define FAMILY_PASS W, age, S, slot_age, data, off, cnt, k, dim, mode, hungarian, alpha, reg, lr
+void family_snapshot(FAMILY_ARGS, at::Tensor sender, at::Tensor slot) {
+    check_idx(sender); check_idx(slot);
+    c10::cuda::CUDAGuard guard(W.device());
+    launch_family_snapshot(family_view(FAMILY_PASS), sender.data_ptr<int>(), slot.data_ptr<int>(), (int)sender.numel(),
+                           cur_stream());
+    GB_LAUNCH_CHECK();
+}
+void kmeans_bank_deliver(FAMILY_ARGS, at::Tensor recv, at::Tensor slot) {
+    check_idx(recv); check_idx(slot);
+    TORCH_CHECK(k * dim <= W.size(1), "kmeans bank: row narrower than k * dim");
+    c10::cuda::CUDAGuard guard(W.device());
+    TORCH_CHECK(launch_kmeans_bank_deliver(family_view(FAMILY_PASS), recv.data_ptr<int>(), slot.data_ptr<int>(),
+                                           (int)recv.numel(), cur_stream()),
+                "kmeans bank: 1 <= k <= ", kFamilyMaxK, " (hungarian matching: k <= 8)");
+    GB_LAUNCH_CHECK();
+}
+at::Tensor kmeans_bank_eval(FAMILY_ARGS, at::Tensor nodes, at::Tensor Xte, at::Tensor yte, int64_t n_true) {
+    check_idx(nodes); check_row(Xte, "Xte");
+    TORCH_CHECK(yte.is_cuda() && yte.scalar_type() == at::kLong && yte.is_contiguous() && yte.numel() == Xte.size(0));
+    TORCH_CHECK(Xte.numel() == Xte.size(0) * dim);
+    c10::cuda::CUDAGuard guard(W.device());
+    auto ct = at::zeros({nodes.numel(), n_true, k}, W.options().dtype(at::kInt));
+    launch_kmeans_bank_eval(family_view(FAMILY_PASS), nodes.data_ptr<int>(), (int)nodes.numel(), Xte.data_ptr<float>(),
+                            yte.data_ptr<int64_t>(), (int)Xte.size(0), (int)n_true, ct.data_ptr<int>(), cur_stream());
+    GB_LAUNCH_CHECK();
+    return ct;
+}
+void mf_bank_deliver(FAMILY_ARGS, at::Tensor recv, at::Tensor slot) {
+    check_idx(recv); check_idx(slot);
+    TORCH_CHECK(dim * k + dim + k + 1 <= W.size(1), "mf bank: row narrower than [Y | c | X | b]");
+    c10::cuda::CUDAGuard guard(W.device());
+    TORCH_CHECK(launch_mf_bank_deliver(family_view(FAMILY_PASS), recv.data_ptr<int>(), slot.data_ptr<int>(),
+                                       (int)recv.numel(), cur_stream()), "mf bank: rank <= 128 supported");
+    GB_LAUNCH_CHECK();
+}
+at::Tensor mf_bank_eval(FAMILY_ARGS, at::Tensor nodes, at::Tensor te, at::Tensor te_off, at::Tensor te_cnt) {
+    check_idx(nodes); check_idx(te_cnt);
+    TORCH_CHECK(te.is_cuda() && te.scalar_type() == at::kFloat && te.is_contiguous());
+    TORCH_CHECK(te_off.is_cuda() && te_off.scalar_type() == at::kLong && te_off.numel() == W.size(0) &&
+                te_cnt.numel() == W.size(0));
+    c10::cuda::CUDAGuard guard(W.device());
+    auto sse = at::empty({nodes.numel()}, W.options());
+    launch_mf_bank_eval(family_view(FAMILY_PASS), nodes.data_ptr<int>(), (int)nodes.numel(), te.data_ptr<float>(),
+                        te_off.data_ptr<int64_t>(), te_cnt.data_ptr<int>(), sse.data_ptr<float>(), cur_stream());
+    GB_LAUNCH_CHECK();
+    return sse;
+}
+
 // ---- multi-process runtime: CUDA-IPC arenas and cross-GPU flags -----------------------------------------
 // One process per GPU (torch.distributed only exchanges the 64-byte IPC handles).  Each rank
 // cudaMalloc's its arena, exports it and maps every peer's arena; a peer row is then a device
@@ -601,6 +671,11 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
           py::arg("item_mode") = py::none());
     m.def("bank_update", &gb::bank_update);
     m.def("bank_scores", &gb::bank_scores);
+    m.def("family_snapshot", &gb::family_snapshot);
+    m.def("kmeans_bank_deliver", &gb::kmeans_bank_deliver);
+    m.def("kmeans_bank_eval", &gb::kmeans_bank_eval);
+    m.def("mf_bank_deliver", &gb::mf_bank_deliver);
+    m.def("mf_bank_eval", &gb::mf_bank_eval);
     m.def("ipc_alloc", &gb::ipc_alloc);
     m.def("ipc_free", &gb::ipc_free);
     m.def("ipc_get_handle", &gb::ipc_get_handle);

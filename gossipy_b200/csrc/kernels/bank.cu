@@ -225,6 +225,7 @@ void preload_bank() {
     cudaFuncGetAttributes(&a, bank_update_kernel<2>); cudaFuncGetAttributes(&a, bank_update_kernel<4>);
     cudaFuncGetAttributes(&a, bank_update_kernel<8>); cudaFuncGetAttributes(&a, bank_update_kernel<32>);
     cudaFuncGetAttributes(&a, bank_scores_kernel);
+    preload_bank_families();
 }
 
 }  // namespace gb

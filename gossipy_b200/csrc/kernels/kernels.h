@@ -158,6 +158,32 @@ void launch_bank_scores(const BankView& b, const int* nodes, int n_nodes, const 
                         cudaStream_t st);
 void preload_bank();
 
+// ---- bank_families.cu: many k-means / matrix-factorisation nodes per launch (one CTA per work item) ----------------
+constexpr int kFamilyMaxK = 64;          // k-means: most centroids per model
+struct FamilyBankView {
+    float* W; long long* age;            // live models [N][Dp] and their ages
+    float* S; long long* slot_age;       // in-flight snapshots [slots][Dp]
+    int Dp;
+    const float* data;                   // local data, concatenated: k-means samples [*][dim], MF ratings [*][2] (item, r)
+    const int64_t* off; const int* cnt;  // node -> first sample / rating, number of them
+    int k, dim;                          // k-means: k centroids of dim floats; MF: rank k, dim = number of items
+    int mode;                            // CreateModelMode value (1 UPDATE, 2 MERGE_UPDATE, 3 UPDATE_MERGE, 4 PASS)
+    int hungarian;                       // k-means: optimal centroid matching before the merge (k <= 8)
+    float alpha;                         // k-means: EMA step
+    float reg, lr;                       // MF: L2 regularisation, learning rate
+};
+// S[slot] = W[sender]: rows of up to 1024 floats go through bank.cu's warp-per-item kernel, wider ones one CTA per item
+void launch_family_snapshot(const FamilyBankView& b, const int* sender, const int* slot, int n, cudaStream_t st);
+bool launch_kmeans_bank_deliver(const FamilyBankView& b, const int* recv, const int* slot, int n, cudaStream_t st);
+// ct [n_nodes][n_true][k] int32, zero on entry
+void launch_kmeans_bank_eval(const FamilyBankView& b, const int* nodes, int n_nodes, const float* Xte, const int64_t* yte,
+                             int n_te, int n_true, int* ct, cudaStream_t st);
+bool launch_mf_bank_deliver(const FamilyBankView& b, const int* recv, const int* slot, int n, cudaStream_t st);
+// sse [n_nodes]: squared error summed over each node's own test ratings te[te_off[node] ..][2]
+void launch_mf_bank_eval(const FamilyBankView& b, const int* nodes, int n_nodes, const float* te, const int64_t* te_off,
+                         const int* te_cnt, float* sse, cudaStream_t st);
+void preload_bank_families();
+
 int sm_count();
 // load every kernel of the extension on the current device (see merge.cu: preload_merge)
 void preload_merge(); void preload_optim(); void preload_small(); void preload_eval();

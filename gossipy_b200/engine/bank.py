@@ -19,6 +19,12 @@ only events that touch *different* nodes are executed together.  Used by
 ``GossipSimulator`` when ``engine="native"`` and the set-up is bankable (plain ``GossipNode``s, one
 shared AdaLine/Pegasos handler configuration, global evaluation set); the handlers' rows and ages
 are written back when the run ends, so the object API sees the same final state.
+
+The model-agnostic part (slot pool, waves, the phases of ``run_round``, checkpoint export / import) is
+:class:`_SlotBank`.  Two more families share it on one rank (``csrc/kernels/bank_families.cu``, one CTA per work
+item): :class:`KMeansBank` (``KMeansHandler``, ``main_berta_2014.py``: 4 601 nodes) and :class:`MFBank`
+(``MFModelHandler``, ``main_hegedus_2020.py``: 6 040 users, rows of ~22 k floats, per-user evaluation).
+:func:`make_bank` picks the bank of a simulation.
 """
 from __future__ import annotations
 
@@ -49,10 +55,12 @@ def close_all() -> None:
 
 
 def bankable(sim) -> Optional[str]:
-    """``None`` if :class:`LinearBank` can execute ``sim``; otherwise the reason it cannot."""
-    from ..model.handler import AdaLineHandler
+    """``None`` if a bank (:func:`make_bank`) can execute ``sim``; otherwise the reason it cannot."""
+    from ..model.handler import AdaLineHandler, KMeansHandler, MFModelHandler
     from ..node import CacheNeighNode, GossipNode, PassThroughNode
     from ..parallel import runtime as prt
+    if isinstance(list(sim.nodes.values())[0].model_handler, (KMeansHandler, MFModelHandler)):
+        return _family_bankable(sim)
     if prt.active() and prt.transport() != "p2p":
         return "several ranks without shared memory"
     if prt.active() and prt.world() > 16:
@@ -60,7 +68,7 @@ def bankable(sim) -> Optional[str]:
     nodes = list(sim.nodes.values())
     h0 = nodes[0].model_handler
     if not isinstance(h0, AdaLineHandler):
-        return "handler is not AdaLine/Pegasos"
+        return "handler is not AdaLine/Pegasos/KMeans/MF"
     cls = type(nodes[0])
     if cls in (PassThroughNode, CacheNeighNode) and not getattr(nodes[0], "_keyed_draws", False):
         return "node-side draws from the host stream"
@@ -81,7 +89,228 @@ def bankable(sim) -> Optional[str]:
     return None
 
 
-class LinearBank:
+class _SlotBank:
+    """What every bank shares, whatever its model: the snapshot slot pool (``S[slots, Dp]``, ``slot_age``, a stack of
+    free slots, ``slot_map`` from message id to slot), the grouping of a tick's deliveries into conflict-free waves,
+    the phase structure of ``run_round`` and the export / import / drop of the messages on the wire (checkpoints).
+    A subclass owns its row layout and data and implements ``_snapshot``, ``_deliver``, ``evaluate`` and
+    ``writeback``."""
+
+    multi = False               # several ranks (LinearBank only)
+    world, rank = 1, 0
+    passthrough = cacheneigh = False
+    eval_on_user = False        # evaluations are reported as per-node (True) or global (False) results
+
+    def _init_slots(self, cap: int) -> None:
+        """Single-rank slot pool of ``cap`` rows (grows on demand, see ``_alloc``)."""
+        self.cap = cap
+        self.S = torch.zeros(self.cap, self.Dp, dtype=torch.float32, device=self.device)
+        self.slot_age = torch.zeros(self.cap, dtype=torch.int64, device=self.device)
+        self.free = np.arange(self.cap - 1, -1, -1, dtype=np.int64)   # stack of free slots
+        self.n_free = self.cap
+
+    def _item_modes(self, recvs: np.ndarray, senders: np.ndarray, slots: np.ndarray) -> Optional[np.ndarray]:
+        return None
+
+    def _idx(self, a) -> torch.Tensor:
+        arr = np.asarray(a, dtype=np.int32)
+        if _PINNED_IDX and self.device.type == "cuda" and arr.size:
+            # a pageable host -> device copy blocks the host until the stream has drained, i.e. it serialises host and device
+            # once per launch; through pinned memory the copy is asynchronous (the caching host allocator keeps the staging
+            # block alive until the copy has run).  Written after the last GPU session: opt-in (GOSSIPY_BANK_PINNED_IDX=1)
+            return torch.from_numpy(np.ascontiguousarray(arr)).pin_memory().to(self.device, non_blocking=True)
+        return torch.as_tensor(arr, device=self.device)
+
+    # -- one round ----------------------------------------------------------------------------------
+    def _alloc(self, k: int) -> np.ndarray:
+        if self.n_free < k:
+            grow = max(self.cap, k)
+            self.S = torch.cat([self.S, torch.zeros(grow, self.Dp, dtype=torch.float32, device=self.device)])
+            self.slot_age = torch.cat([self.slot_age, torch.zeros(grow, dtype=torch.int64, device=self.device)])
+            self.free = np.concatenate([self.free[:self.n_free], np.arange(self.cap, self.cap + grow, dtype=np.int64)])
+            self.n_free += grow
+            self.cap += grow
+        out = self.free[self.n_free - k:self.n_free].copy()
+        self.n_free -= k
+        return out
+
+    def _release(self, slots: np.ndarray) -> None:
+        slots = slots[slots >= 0]
+        k = slots.size
+        if k:
+            if self.n_free + k > self.free.size:
+                self.free = np.concatenate([self.free, np.empty(self.n_free + k - self.free.size, dtype=np.int64)])
+            self.free[self.n_free:self.n_free + k] = slots
+            self.n_free += k
+
+    @staticmethod
+    def _waves(recv: np.ndarray) -> List[np.ndarray]:
+        """Indices of ``recv`` grouped so that wave k holds the k-th occurrence of every receiver."""
+        if recv.size == 0:
+            return []
+        order = np.argsort(recv, kind="stable")
+        sorted_r = recv[order]
+        first = np.r_[True, sorted_r[1:] != sorted_r[:-1]]
+        start = np.maximum.accumulate(np.where(first, np.arange(recv.size), 0))
+        rank = np.empty(recv.size, dtype=np.int64)
+        rank[order] = np.arange(recv.size) - start
+        return [np.flatnonzero(rank == k) for k in range(int(rank.max()) + 1)]
+
+    def run_round(self, events: np.ndarray, C: Any) -> Tuple[List[int], Dict[str, int]]:
+        """Execute one round's event list; returns (nodes to evaluate, message counters)."""
+        if self.multi:
+            return self._run_round_multi(events, C)
+        kind, tick, a, b, slot, aux = (events[:, i] for i in range(6))
+        counters = {"sent": 0, "sent_size": 0, "failed": 0}
+        evals: List[int] = []
+        if events.shape[0] == 0:
+            return evals, counters
+        bounds = np.flatnonzero(np.r_[True, tick[1:] != tick[:-1], True])
+        for lo, hi in zip(bounds[:-1], bounds[1:]):
+            k, ea, eb, es, ex = kind[lo:hi], a[lo:hi], b[lo:hi], slot[lo:hi], aux[lo:hi]
+            # ---- phase A: sends (a snapshot per model-carrying message) -------------------------------
+            m = k == C.EV_SEND
+            if m.any():
+                senders, mids, mtypes = ea[m], es[m], ex[m]
+                carries = mtypes != 2                                   # 2 = PULL request
+                if self.cacheneigh:                                     # consume one cached model before the snapshot
+                    cn_nodes, cn_slots = self._cn_pick(senders, mtypes)
+                    self._deliver(cn_nodes, cn_slots)
+                    self._release(cn_slots)
+                slots = np.full(senders.size, -1, dtype=np.int64)
+                slots[carries] = self._alloc(int(carries.sum()))
+                self.slot_map[mids % _RING] = slots
+                self._snapshot(senders, slots)
+                counters["sent"] += int(senders.size)
+                counters["sent_size"] += int(carries.sum()) * self.size_model + int((~carries).sum())
+            # ---- phase B: deliveries (+ the replies they trigger), conflict-free waves ---------------
+            m = k == C.EV_DELIVER
+            if m.any():
+                origin, recv, mids = ea[m], eb[m], es[m]
+                # replies: EV_REPLY_SEND(slot = request id, aux = reply id) follows its delivery
+                rs = k == C.EV_REPLY_SEND
+                req_ids, rep_ids = es[rs], ex[rs]
+                has_reply = np.isin(mids, req_ids) if req_ids.size else np.zeros(mids.size, dtype=bool)
+                rep_of = None
+                if req_ids.size:
+                    srt = np.argsort(req_ids)
+                    pos_in = np.searchsorted(req_ids[srt], mids[has_reply])
+                    rep_of = np.full(mids.size, -1, dtype=np.int64)
+                    rep_of[has_reply] = rep_ids[srt][pos_in]
+                for idx in ([np.arange(recv.size)] if self.cacheneigh else self._waves(recv)):
+                    r_w, mid_w = recv[idx], mids[idx]
+                    s_w = self.slot_map[mid_w % _RING].copy()
+                    if self.cacheneigh:                                 # only stored (newest per sender)
+                        self._release(self._cn_store(r_w, origin[idx], s_w))
+                    else:
+                        self._deliver(r_w, s_w, self._item_modes(r_w, origin[idx], s_w))
+                        self._release(s_w)
+                    if rep_of is not None:
+                        sel = has_reply[idx]
+                        if sel.any():
+                            rslots = self._alloc(int(sel.sum()))
+                            self.slot_map[rep_of[idx][sel] % _RING] = rslots
+                            self._snapshot(r_w[sel], rslots)
+            # ---- phase C: replies delivered ------------------------------------------------------------
+            m = k == C.EV_REPLY_DELIVER
+            if m.any():
+                recv, repl, mids = ea[m], eb[m], es[m]
+                counters["sent"] += int(recv.size)
+                counters["sent_size"] += int(recv.size) * self.size_model
+                for idx in ([np.arange(recv.size)] if self.cacheneigh else self._waves(recv)):
+                    s_w = self.slot_map[mids[idx] % _RING].copy()
+                    if self.cacheneigh:
+                        self._release(self._cn_store(recv[idx], repl[idx], s_w))
+                    else:
+                        self._deliver(recv[idx], s_w, self._item_modes(recv[idx], repl[idx], s_w))
+                        self._release(s_w)
+            # ---- losses: free the snapshot -------------------------------------------------------------
+            m = k == C.EV_DROP
+            if m.any():
+                counters["failed"] += int(m.sum())
+                dropped = self.slot_map[es[m] % _RING].copy()
+                self.slot_map[es[m] % _RING] = -1
+                self._release(dropped)
+            m = k == C.EV_EVAL
+            if m.any():
+                evals.extend(ea[m].tolist())
+        return evals, counters
+
+    # -- checkpointing -----------------------------------------------------------------------------
+    def export_inflight(self, message_ids: List[int], receivers: Optional[List[int]] = None) -> Dict[str, Any]:
+        """Snapshots of the messages that are still on the wire (ids from the scheduler's queues; ``receivers`` = the
+        node each of them travels to).  Several ranks: a snapshot lives in the bank of its receiver's rank, so every
+        rank contributes its part and all ranks end up with the complete set (every rank writes a full checkpoint)."""
+        ids = np.asarray(message_ids, dtype=np.int64)
+        recv = np.asarray(receivers if receivers is not None else np.zeros(ids.size), dtype=np.int64)
+        slots = self.slot_map[ids % _RING] if ids.size else np.zeros(0, dtype=np.int64)
+        keep = slots >= 0
+        ids, slots, recv = ids[keep], slots[keep], recv[keep]
+        ent = []
+        if self.cacheneigh:                 # models waiting in the neighbour caches are state as well
+            ent = [(n, s, sl) for n, cache in enumerate(self.cn_cache) for s, sl in sorted(cache.items())]
+        if self.multi:
+            return self._export_inflight_multi(ids, slots, recv, ent)
+        idx = torch.as_tensor(slots, dtype=torch.int64, device=self.device)
+        out = {"ids": ids, "receivers": recv, "rows": self.S[idx].cpu(), "ages": self.slot_age[idx].cpu()}
+        if self.cacheneigh:
+            cidx = torch.as_tensor([e[2] for e in ent], dtype=torch.int64, device=self.device)
+            out["cn"] = {"nodes": [e[0] for e in ent], "senders": [e[1] for e in ent],
+                         "rows": self.S[cidx].cpu(), "ages": self.slot_age[cidx].cpu()}
+        return out
+
+    def _place(self, dst_nodes: np.ndarray, rows: torch.Tensor, ages: torch.Tensor) -> Tuple[np.ndarray, np.ndarray]:
+        """Slots for restored snapshots that travel to / are cached at ``dst_nodes``; returns (slots, ranks)."""
+        k = int(dst_nodes.size)
+        if not self.multi:
+            slots = self._alloc(k)
+            idx = torch.as_tensor(slots, dtype=torch.int64, device=self.device)
+            self.S[idx] = rows.to(self.device)
+            self.slot_age[idx] = ages.to(self.device)
+            return slots, np.zeros(k, dtype=np.int64)
+        ranks = self.owner[dst_nodes]
+        slots = self._alloc_multi(ranks)            # replicated bookkeeping; every rank fills the slots of its own bank
+        mine = ranks == self.rank
+        if mine.any():
+            idx = torch.as_tensor(slots[mine], dtype=torch.int64, device=self.device)
+            sel = torch.as_tensor(np.flatnonzero(mine), dtype=torch.int64)
+            self.S[idx] = rows[sel].to(self.device)
+            self.slot_age[idx] = ages[sel].to(self.device)
+        return slots, ranks
+
+    def import_inflight(self, st: Dict[str, Any]) -> None:
+        cn = st.get("cn")
+        if cn is not None and len(cn["nodes"]):
+            slots, _ = self._place(np.asarray(cn["nodes"], dtype=np.int64), cn["rows"], cn["ages"])
+            for n, s, sl in zip(cn["nodes"], cn["senders"], slots.tolist()):
+                self.cn_cache[n][s] = sl
+        ids = np.asarray(st["ids"], dtype=np.int64)
+        if ids.size == 0:
+            return
+        recv = np.asarray(st.get("receivers", np.zeros(ids.size)), dtype=np.int64)
+        slots, ranks = self._place(recv, st["rows"], st["ages"])
+        self.slot_map[ids % _RING] = slots
+        if self.multi:
+            self.slot_rank[ids % _RING] = ranks
+
+    def drop_inflight(self) -> None:
+        """A fresh ``start`` forgets the messages on the wire: every slot that is not a cached model (cache-neighbour nodes:
+        node state) goes back to its pool.  Replicated bookkeeping, no device work."""
+        cached = [dict() for _ in range(self.world)]
+        if self.cacheneigh:
+            for node, cache in enumerate(self.cn_cache):
+                for sl in cache.values():
+                    cached[int(self.owner[node]) if self.multi else 0][int(sl)] = True
+        self.slot_map[:] = -1
+        if self.multi:
+            for r in range(self.world):
+                free = np.asarray([s for s in range(self.cap - 1, -1, -1) if s not in cached[r]], dtype=np.int64)
+                self.free_r[r], self.n_free_r[r], self.pending_r[r] = free, int(free.size), []
+        else:
+            self.free = np.asarray([s for s in range(self.cap - 1, -1, -1) if s not in cached[0]], dtype=np.int64)
+            self.n_free = int(self.free.size)
+
+class LinearBank(_SlotBank):
     def __init__(self, sim) -> None:
         from ..model.handler import PegasosHandler
         self.sim = sim
@@ -131,10 +360,7 @@ class LinearBank:
         if self.multi:
             self._init_shared_slots()
         else:
-            self.S = torch.zeros(self.cap, self.Dp, dtype=torch.float32, device=dev)
-            self.slot_age = torch.zeros(self.cap, dtype=torch.int64, device=dev)
-            self.free = np.arange(self.cap - 1, -1, -1, dtype=np.int64)   # stack of free slots
-            self.n_free = self.cap
+            self._init_slots(self.cap)
         # evaluation set
         self.Xte = self.yte = None
         if sim.data_dispatcher.has_test():
@@ -342,15 +568,6 @@ class LinearBank:
         return (self.W, self.age, self.S, self.slot_age, self.X, self.y, self.off, self.cnt, self.D, self.kind,
                 self.mode, self.lr)
 
-    def _idx(self, a) -> torch.Tensor:
-        arr = np.asarray(a, dtype=np.int32)
-        if _PINNED_IDX and self.device.type == "cuda" and arr.size:
-            # a pageable host -> device copy blocks the host until the stream has drained, i.e. it serialises host and device
-            # once per launch; through pinned memory the copy is asynchronous (the caching host allocator keeps the staging
-            # block alive until the copy has run).  Written after the last GPU session: opt-in (GOSSIPY_BANK_PINNED_IDX=1)
-            return torch.from_numpy(np.ascontiguousarray(arr)).pin_memory().to(self.device, non_blocking=True)
-        return torch.as_tensor(arr, device=self.device)
-
     def _snapshot(self, senders, slots) -> None:
         if len(senders) == 0:
             return
@@ -445,121 +662,7 @@ class LinearBank:
         idx = torch.as_tensor(np.asarray(nodes), dtype=torch.int64)
         return self.W[idx, :self.D] @ self.Xte.t()
 
-    # -- one round ----------------------------------------------------------------------------------
-    def _alloc(self, k: int) -> np.ndarray:
-        if self.n_free < k:
-            grow = max(self.cap, k)
-            self.S = torch.cat([self.S, torch.zeros(grow, self.Dp, dtype=torch.float32, device=self.device)])
-            self.slot_age = torch.cat([self.slot_age, torch.zeros(grow, dtype=torch.int64, device=self.device)])
-            self.free = np.concatenate([self.free[:self.n_free], np.arange(self.cap, self.cap + grow, dtype=np.int64)])
-            self.n_free += grow
-            self.cap += grow
-        out = self.free[self.n_free - k:self.n_free].copy()
-        self.n_free -= k
-        return out
-
-    def _release(self, slots: np.ndarray) -> None:
-        slots = slots[slots >= 0]
-        k = slots.size
-        if k:
-            if self.n_free + k > self.free.size:
-                self.free = np.concatenate([self.free, np.empty(self.n_free + k - self.free.size, dtype=np.int64)])
-            self.free[self.n_free:self.n_free + k] = slots
-            self.n_free += k
-
-    @staticmethod
-    def _waves(recv: np.ndarray) -> List[np.ndarray]:
-        """Indices of ``recv`` grouped so that wave k holds the k-th occurrence of every receiver."""
-        if recv.size == 0:
-            return []
-        order = np.argsort(recv, kind="stable")
-        sorted_r = recv[order]
-        first = np.r_[True, sorted_r[1:] != sorted_r[:-1]]
-        start = np.maximum.accumulate(np.where(first, np.arange(recv.size), 0))
-        rank = np.empty(recv.size, dtype=np.int64)
-        rank[order] = np.arange(recv.size) - start
-        return [np.flatnonzero(rank == k) for k in range(int(rank.max()) + 1)]
-
-    def run_round(self, events: np.ndarray, C: Any) -> Tuple[List[int], Dict[str, int]]:
-        """Execute one round's event list; returns (nodes to evaluate, message counters)."""
-        if self.multi:
-            return self._run_round_multi(events, C)
-        kind, tick, a, b, slot, aux = (events[:, i] for i in range(6))
-        counters = {"sent": 0, "sent_size": 0, "failed": 0}
-        evals: List[int] = []
-        if events.shape[0] == 0:
-            return evals, counters
-        bounds = np.flatnonzero(np.r_[True, tick[1:] != tick[:-1], True])
-        for lo, hi in zip(bounds[:-1], bounds[1:]):
-            k, ea, eb, es, ex = kind[lo:hi], a[lo:hi], b[lo:hi], slot[lo:hi], aux[lo:hi]
-            # ---- phase A: sends (a snapshot per model-carrying message) -------------------------------
-            m = k == C.EV_SEND
-            if m.any():
-                senders, mids, mtypes = ea[m], es[m], ex[m]
-                carries = mtypes != 2                                   # 2 = PULL request
-                if self.cacheneigh:                                     # consume one cached model before the snapshot
-                    cn_nodes, cn_slots = self._cn_pick(senders, mtypes)
-                    self._deliver(cn_nodes, cn_slots)
-                    self._release(cn_slots)
-                slots = np.full(senders.size, -1, dtype=np.int64)
-                slots[carries] = self._alloc(int(carries.sum()))
-                self.slot_map[mids % _RING] = slots
-                self._snapshot(senders, slots)
-                counters["sent"] += int(senders.size)
-                counters["sent_size"] += int(carries.sum()) * self.size_model + int((~carries).sum())
-            # ---- phase B: deliveries (+ the replies they trigger), conflict-free waves ---------------
-            m = k == C.EV_DELIVER
-            if m.any():
-                origin, recv, mids = ea[m], eb[m], es[m]
-                # replies: EV_REPLY_SEND(slot = request id, aux = reply id) follows its delivery
-                rs = k == C.EV_REPLY_SEND
-                req_ids, rep_ids = es[rs], ex[rs]
-                has_reply = np.isin(mids, req_ids) if req_ids.size else np.zeros(mids.size, dtype=bool)
-                rep_of = None
-                if req_ids.size:
-                    srt = np.argsort(req_ids)
-                    pos_in = np.searchsorted(req_ids[srt], mids[has_reply])
-                    rep_of = np.full(mids.size, -1, dtype=np.int64)
-                    rep_of[has_reply] = rep_ids[srt][pos_in]
-                for idx in ([np.arange(recv.size)] if self.cacheneigh else self._waves(recv)):
-                    r_w, mid_w = recv[idx], mids[idx]
-                    s_w = self.slot_map[mid_w % _RING].copy()
-                    if self.cacheneigh:                                 # only stored (newest per sender)
-                        self._release(self._cn_store(r_w, origin[idx], s_w))
-                    else:
-                        self._deliver(r_w, s_w, self._item_modes(r_w, origin[idx], s_w))
-                        self._release(s_w)
-                    if rep_of is not None:
-                        sel = has_reply[idx]
-                        if sel.any():
-                            rslots = self._alloc(int(sel.sum()))
-                            self.slot_map[rep_of[idx][sel] % _RING] = rslots
-                            self._snapshot(r_w[sel], rslots)
-            # ---- phase C: replies delivered ------------------------------------------------------------
-            m = k == C.EV_REPLY_DELIVER
-            if m.any():
-                recv, repl, mids = ea[m], eb[m], es[m]
-                counters["sent"] += int(recv.size)
-                counters["sent_size"] += int(recv.size) * self.size_model
-                for idx in ([np.arange(recv.size)] if self.cacheneigh else self._waves(recv)):
-                    s_w = self.slot_map[mids[idx] % _RING].copy()
-                    if self.cacheneigh:
-                        self._release(self._cn_store(recv[idx], repl[idx], s_w))
-                    else:
-                        self._deliver(recv[idx], s_w, self._item_modes(recv[idx], repl[idx], s_w))
-                        self._release(s_w)
-            # ---- losses: free the snapshot -------------------------------------------------------------
-            m = k == C.EV_DROP
-            if m.any():
-                counters["failed"] += int(m.sum())
-                dropped = self.slot_map[es[m] % _RING].copy()
-                self.slot_map[es[m] % _RING] = -1
-                self._release(dropped)
-            m = k == C.EV_EVAL
-            if m.any():
-                evals.extend(ea[m].tolist())
-        return evals, counters
-
+    # -- one round, several ranks -----------------------------------------------------------------------
     def _run_round_multi(self, events: np.ndarray, C: Any) -> Tuple[List[int], Dict[str, int]]:
         """``run_round`` with the nodes spread over several ranks: same phases, every rank launches the work of its own
         nodes; a phase that pushed snapshots across ranks ends with a barrier."""
@@ -703,30 +806,7 @@ class LinearBank:
         return [{"accuracy": float(acc[e]), "precision": float(prec[e]), "recall": float(recl[e]),
                  "f1_score": float(f1[e]), "auc": float(auc[e])} for e in range(E)]
 
-    # -- synchronise the object API -----------------------------------------------------------------------
-    # -- checkpointing -----------------------------------------------------------------------------
-    def export_inflight(self, message_ids: List[int], receivers: Optional[List[int]] = None) -> Dict[str, Any]:
-        """Snapshots of the messages that are still on the wire (ids from the scheduler's queues; ``receivers`` = the
-        node each of them travels to).  Several ranks: a snapshot lives in the bank of its receiver's rank, so every
-        rank contributes its part and all ranks end up with the complete set (every rank writes a full checkpoint)."""
-        ids = np.asarray(message_ids, dtype=np.int64)
-        recv = np.asarray(receivers if receivers is not None else np.zeros(ids.size), dtype=np.int64)
-        slots = self.slot_map[ids % _RING] if ids.size else np.zeros(0, dtype=np.int64)
-        keep = slots >= 0
-        ids, slots, recv = ids[keep], slots[keep], recv[keep]
-        ent = []
-        if self.cacheneigh:                 # models waiting in the neighbour caches are state as well
-            ent = [(n, s, sl) for n, cache in enumerate(self.cn_cache) for s, sl in sorted(cache.items())]
-        if self.multi:
-            return self._export_inflight_multi(ids, slots, recv, ent)
-        idx = torch.as_tensor(slots, dtype=torch.int64, device=self.device)
-        out = {"ids": ids, "receivers": recv, "rows": self.S[idx].cpu(), "ages": self.slot_age[idx].cpu()}
-        if self.cacheneigh:
-            cidx = torch.as_tensor([e[2] for e in ent], dtype=torch.int64, device=self.device)
-            out["cn"] = {"nodes": [e[0] for e in ent], "senders": [e[1] for e in ent],
-                         "rows": self.S[cidx].cpu(), "ages": self.slot_age[cidx].cpu()}
-        return out
-
+    # -- checkpointing, several ranks --------------------------------------------------------------------
     def _export_inflight_multi(self, ids: np.ndarray, slots: np.ndarray, recv: np.ndarray, ent: List) -> Dict[str, Any]:
         import torch.distributed as dist
         self._barrier()                     # everything pushed towards this rank has landed
@@ -751,57 +831,6 @@ class LinearBank:
                          "rows": torch.cat([q["cn_rows"] for q in parts]), "ages": torch.cat([q["cn_ages"] for q in parts])}
         return out
 
-    def _place(self, dst_nodes: np.ndarray, rows: torch.Tensor, ages: torch.Tensor) -> Tuple[np.ndarray, np.ndarray]:
-        """Slots for restored snapshots that travel to / are cached at ``dst_nodes``; returns (slots, ranks)."""
-        k = int(dst_nodes.size)
-        if not self.multi:
-            slots = self._alloc(k)
-            idx = torch.as_tensor(slots, dtype=torch.int64, device=self.device)
-            self.S[idx] = rows.to(self.device)
-            self.slot_age[idx] = ages.to(self.device)
-            return slots, np.zeros(k, dtype=np.int64)
-        ranks = self.owner[dst_nodes]
-        slots = self._alloc_multi(ranks)            # replicated bookkeeping; every rank fills the slots of its own bank
-        mine = ranks == self.rank
-        if mine.any():
-            idx = torch.as_tensor(slots[mine], dtype=torch.int64, device=self.device)
-            sel = torch.as_tensor(np.flatnonzero(mine), dtype=torch.int64)
-            self.S[idx] = rows[sel].to(self.device)
-            self.slot_age[idx] = ages[sel].to(self.device)
-        return slots, ranks
-
-    def import_inflight(self, st: Dict[str, Any]) -> None:
-        cn = st.get("cn")
-        if cn is not None and len(cn["nodes"]):
-            slots, _ = self._place(np.asarray(cn["nodes"], dtype=np.int64), cn["rows"], cn["ages"])
-            for n, s, sl in zip(cn["nodes"], cn["senders"], slots.tolist()):
-                self.cn_cache[n][s] = sl
-        ids = np.asarray(st["ids"], dtype=np.int64)
-        if ids.size == 0:
-            return
-        recv = np.asarray(st.get("receivers", np.zeros(ids.size)), dtype=np.int64)
-        slots, ranks = self._place(recv, st["rows"], st["ages"])
-        self.slot_map[ids % _RING] = slots
-        if self.multi:
-            self.slot_rank[ids % _RING] = ranks
-
-    def drop_inflight(self) -> None:
-        """A fresh ``start`` forgets the messages on the wire: every slot that is not a cached model (cache-neighbour nodes:
-        node state) goes back to its pool.  Replicated bookkeeping, no device work."""
-        cached = [dict() for _ in range(self.world)]
-        if self.cacheneigh:
-            for node, cache in enumerate(self.cn_cache):
-                for sl in cache.values():
-                    cached[int(self.owner[node]) if self.multi else 0][int(sl)] = True
-        self.slot_map[:] = -1
-        if self.multi:
-            for r in range(self.world):
-                free = np.asarray([s for s in range(self.cap - 1, -1, -1) if s not in cached[r]], dtype=np.int64)
-                self.free_r[r], self.n_free_r[r], self.pending_r[r] = free, int(free.size), []
-        else:
-            self.free = np.asarray([s for s in range(self.cap - 1, -1, -1) if s not in cached[0]], dtype=np.int64)
-            self.n_free = int(self.free.size)
-
     def writeback(self) -> None:
         W = self.W[:, :self.D]
         age = self.age
@@ -823,3 +852,309 @@ class LinearBank:
                 node._cn_draws = int(self.cn_count[i])
         if self.multi:
             self.age.copy_(age)
+
+
+# -- k-means and matrix factorisation ------------------------------------------------------------------------------
+_SLOT_BYTES = 256 << 20     # first slot-pool allocation of the family banks (the pool grows on demand)
+
+
+def _family_bankable(sim) -> Optional[str]:
+    """:class:`KMeansBank` / :class:`MFBank`: plain ``GossipNode``s on a ``GossipSimulator``, one rank, one handler
+    configuration.  Under ``reference_compat`` k-means "hungarian" merges like "naive", as ``KMeansHandler`` does then."""
+    from ..model.handler import KMeansHandler, MFModelHandler
+    from ..node import GossipNode
+    from ..parallel import runtime as prt
+    if prt.active():
+        return "several ranks (k-means / MF banks run on one rank)"
+    if type(sim).__name__ != "GossipSimulator":
+        return "simulator variant"
+    nodes = list(sim.nodes.values())
+    h0 = nodes[0].model_handler
+    if isinstance(h0, KMeansHandler):
+        key = lambda h: (type(h), h.k, h.dim, h.alpha, h.matching, h.mode)     # noqa: E731
+        if h0.matching == "hungarian" and h0.k > 8:
+            return "hungarian matching with k > 8"
+        if h0.k > 64:
+            return "k-means with k > 64"
+    else:
+        key = lambda h: (type(h), h.k, h.n_items, h.reg, h.lr, h.mode)         # noqa: E731
+        if h0.k > 128:
+            return "matrix factorisation with k > 128"
+    if type(h0) not in (KMeansHandler, MFModelHandler):
+        return "handler subclass"
+    k0 = key(h0)
+    for n in nodes:
+        if type(n) is not GossipNode:
+            return "node class %s" % type(n).__name__
+        if key(n.model_handler) != k0:
+            return "heterogeneous handlers"
+        if isinstance(h0, KMeansHandler) and n.has_test():
+            return "per-node test sets"
+    if h0.mode not in _MODE:
+        return "unsupported mode"
+    if isinstance(h0, KMeansHandler) and not sim.data_dispatcher.has_test():
+        return "no evaluation set"
+    return None
+
+
+def make_bank(sim) -> _SlotBank:
+    """The bank that executes ``sim`` (which :func:`bankable` accepted)."""
+    from ..model.handler import KMeansHandler, MFModelHandler
+    h0 = sim.nodes[min(sim.nodes)].model_handler
+    if isinstance(h0, KMeansHandler):
+        return KMeansBank(sim)
+    if isinstance(h0, MFModelHandler):
+        return MFBank(sim)
+    return LinearBank(sim)
+
+
+def _np(a: Any) -> np.ndarray:
+    return a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a)
+
+
+class _FamilyBank(_SlotBank):
+    """A bank whose rows are exactly the handlers' arena rows (``h._row_numel`` floats), one CTA per work item on a
+    GPU.  Subclasses set up ``data`` / ``off`` / ``cnt`` and implement the delivery and the evaluation."""
+
+    def __init__(self, sim) -> None:
+        self.sim = sim
+        ids = sorted(sim.nodes)
+        self.n = len(ids)
+        h0 = sim.nodes[ids[0]].model_handler
+        self.device = h0.device
+        self.Dp = int(h0._row_numel)
+        self.mode = _MODE[h0.mode]
+        if self.device.type == "cuda":            # the handlers' rows were written on the nodes' streams
+            torch.cuda.synchronize(self.device)
+        self.W = torch.stack([sim.nodes[i].model_handler.row for i in ids]).to(self.device).contiguous()
+        self.age = torch.tensor([int(sim.nodes[i].model_handler.n_updates) for i in ids], dtype=torch.int64,
+                                device=self.device)
+        self.slot_map = np.full(_RING, -1, dtype=np.int64)            # message id (mod ring) -> slot
+        self._init_slots(max(64, min(4 * self.n, _SLOT_BYTES // (4 * self.Dp))))
+        self.size_model = int(h0.get_size())
+
+    @staticmethod
+    def _concat(parts: List[np.ndarray], width: int, device) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        """Per-node arrays [n_i, width] -> (concatenation as fp32, offsets int64, counts int32) on ``device``."""
+        cnt = [int(p.shape[0]) for p in parts]
+        off = np.concatenate([[0], np.cumsum(cnt)[:-1]]).astype(np.int64) if cnt else np.zeros(0, np.int64)
+        flat = np.concatenate(parts).astype(np.float32) if parts else np.zeros((0, width), np.float32)
+        if flat.shape[0] == 0:
+            flat = np.zeros((1, width), np.float32)                     # (a valid pointer for the kernels)
+        return (torch.from_numpy(np.ascontiguousarray(flat.reshape(-1, width))).to(device),
+                torch.from_numpy(off).to(device), torch.tensor(cnt, dtype=torch.int32, device=device))
+
+    def _args(self):
+        return (self.W, self.age, self.S, self.slot_age, self.data, self.off, self.cnt, self.k, self.dim, self.mode,
+                self.hungarian, self.alpha, self.reg, self.lr)
+
+    def _snapshot(self, senders, slots) -> None:
+        if len(senders) == 0:
+            return
+        if self.device.type == "cuda":
+            from ..ops.native import native
+            native().family_snapshot(*self._args(), self._idx(senders), self._idx(slots))
+            ops._count()
+            return
+        s = torch.as_tensor(np.asarray(senders), dtype=torch.int64)
+        d = torch.as_tensor(np.asarray(slots), dtype=torch.int64)
+        keep = d >= 0
+        self.S[d[keep]] = self.W[s[keep]]
+        self.slot_age[d[keep]] = self.age[s[keep]]
+
+    def _deliver(self, recvs, slots, modes=None) -> None:
+        if len(recvs) == 0:
+            return
+        if self.device.type == "cuda":
+            self._deliver_cuda(self._idx(recvs), self._idx(slots))
+            ops._count()
+            return
+        r = torch.as_tensor(np.asarray(recvs), dtype=torch.int64)
+        s = torch.as_tensor(np.asarray(slots), dtype=torch.int64)
+        keep = s >= 0
+        r, s = r[keep], s[keep]
+        if r.numel() == 0:
+            return
+        w, sv = self.W[r].clone(), self.S[s].clone()
+        aw, asn = self.age[r].clone(), self.slot_age[s].clone()
+        if self.mode == 1:                      # UPDATE: adopt the received model (and its age), train it
+            w, aw = sv, asn
+            aw = aw + self._update_cpu(w, r)
+        elif self.mode == 2:                    # MERGE_UPDATE
+            self._merge_cpu(w, sv, aw, asn)
+            aw = aw + self._update_cpu(w, r)
+        elif self.mode == 3:                    # UPDATE_MERGE: both models train on the local data, then merge
+            aw = aw + self._update_cpu(w, r)
+            asn = asn + self._update_cpu(sv, r)
+            self._merge_cpu(w, sv, aw, asn)
+        else:                                   # PASS: adopt untouched, age unchanged
+            w = sv
+        self.W[r] = w
+        self.age[r] = aw
+
+    def evaluate(self, nodes: List[int]) -> List[Dict[str, float]]:
+        if not nodes:
+            return []
+        return self._evaluate(nodes)
+
+    def writeback(self) -> None:
+        W = self.W.cpu() if self.device.type == "cpu" else self.W
+        ages = self.age.cpu().tolist()
+        for i, node in self.sim.nodes.items():
+            h = node.model_handler
+            h.row.copy_(W[i])
+            h.n_updates = int(ages[i])
+            h._version += 1
+        if self.device.type == "cuda":            # the rows are read next on the nodes' own streams
+            torch.cuda.synchronize(self.device)
+
+
+class KMeansBank(_FamilyBank):
+    """Online k-means (``KMeansHandler``): row = the ``k x dim`` centroids, padded; data = every node's local samples,
+    concatenated.  Deliveries: merge 0.5 / 0.5 (naive, or after the optimal centroid matching for "hungarian",
+    k <= 8), local update = the batched EMA step with the last sample per centroid winning.  Evaluation: the NMI of
+    the cluster assignment on the shared evaluation set, one contingency table per node from one launch."""
+
+    def __init__(self, sim) -> None:
+        from .. import GlobalSettings
+        super().__init__(sim)
+        h0 = sim.nodes[min(sim.nodes)].model_handler
+        self.k, self.dim, self.alpha = int(h0.k), int(h0.dim), float(h0.alpha)
+        # (reference_compat: the reference's "hungarian" is the identity assignment, KMeansHandler._merge)
+        self.hungarian = h0.matching == "hungarian" and not GlobalSettings().reference_compat
+        self.reg = self.lr = 0.0
+        parts = [_np(sim.nodes[i].data[0][0]).reshape(-1, self.dim) for i in sorted(sim.nodes)]
+        self.data, self.off, self.cnt = self._concat(parts, self.dim, self.device)
+        Xte, yte = sim.data_dispatcher.get_eval_set()
+        y_host = _np(yte).reshape(-1).astype(np.int64)
+        self.n_true = int(y_host.max()) + 1 if y_host.size else 1
+        self.Xte = torch.as_tensor(_np(Xte), dtype=torch.float32).reshape(-1, self.dim).contiguous().to(self.device)
+        self.yte = torch.from_numpy(y_host).to(self.device)
+
+    def _deliver_cuda(self, recvs: torch.Tensor, slots: torch.Tensor) -> None:
+        from ..ops.native import native
+        native().kmeans_bank_deliver(*self._args(), recvs, slots)
+
+    def _update_cpu(self, w: torch.Tensor, nodes: torch.Tensor) -> torch.Tensor:
+        """In place on the rows ``w`` [B, Dp], vectorised over the nodes (``torch_ref.kmeans_update``); returns the
+        age increments."""
+        B, k, d = w.shape[0], self.k, self.dim
+        C = w[:, :k * d].view(B, k, d)
+        cnt, off = self.cnt[nodes].long(), self.off[nodes]
+        m = int(cnt.max())
+        if m > 0:
+            ar = torch.arange(m)
+            valid = ar[None, :] < cnt[:, None]
+            X = self.data[(off[:, None] + ar[None, :]).clamp(max=self.data.shape[0] - 1)]        # [B, m, d]
+            asg = torch.cdist(X, C, p=2).argmin(dim=2)                                          # [B, m]
+            hit = (asg[:, :, None] == torch.arange(k)[None, None, :]) & valid[:, :, None]       # [B, m, k]
+            winner = torch.where(hit, ar[None, :, None].expand(B, m, k), torch.full_like(hit, -1, dtype=torch.long)).amax(1)
+            sel = winner >= 0
+            xw = X[torch.arange(B)[:, None], winner.clamp(min=0)]                                 # [B, k, d]
+            C.copy_(torch.where(sel[:, :, None], C * (1 - self.alpha) + self.alpha * xw, C))
+        return torch.ones(B, dtype=torch.int64)
+
+    def _merge_cpu(self, w: torch.Tensor, sv: torch.Tensor, aw: torch.Tensor, asn: torch.Tensor) -> None:
+        k, d = self.k, self.dim
+        if not self.hungarian:
+            w.mul_(0.5).add_(sv, alpha=0.5)
+            return
+        from scipy.optimize import linear_sum_assignment
+        for b in range(w.shape[0]):
+            own, theirs = w[b, :k * d].view(k, d), sv[b, :k * d].view(k, d)
+            cols = linear_sum_assignment(torch.cdist(own, theirs).numpy())[1]
+            own.copy_(0.5 * own + 0.5 * theirs[torch.as_tensor(cols)])
+
+    def _evaluate(self, nodes: List[int]) -> List[Dict[str, float]]:
+        from ..ops import metrics
+        k = self.k
+        if self.device.type == "cuda":
+            from ..ops.native import native
+            ct = native().kmeans_bank_eval(*self._args(), self._idx(nodes), self.Xte, self.yte, self.n_true)
+            ops._count()
+            cts = ct.cpu().numpy()
+        else:
+            from ..ops import torch_ref
+            cts = []
+            for i in nodes:
+                pred = torch_ref.kmeans_assign(self.W[i, :k * self.dim].view(k, self.dim), self.Xte)
+                cts.append(torch.bincount(self.yte * k + pred.long(), minlength=self.n_true * k)
+                           .view(self.n_true, k).numpy())
+        return [{"nmi": metrics.nmi_from_contingency(c)} for c in cts]
+
+
+class MFBank(_FamilyBank):
+    """Matrix factorisation (``MFModelHandler``): row = ``[Y (n_items*k) | c (n_items) | X (k) | b (1)]``, padded;
+    data = every node's train ratings (item, rating), concatenated, and its own test ratings likewise.  Deliveries:
+    the item side ``[Y | c]`` merged with the age weights ``a/(2(a+b))``, ``b/(2(a+b))``, then the sequential SGD over
+    the node's ratings.  Evaluation: the RMSE of every evaluated node on its own test ratings (per-node results)."""
+
+    eval_on_user = True
+
+    def __init__(self, sim) -> None:
+        super().__init__(sim)
+        h0 = sim.nodes[min(sim.nodes)].model_handler
+        self.k, self.dim = int(h0.k), int(h0.n_items)
+        self.reg, self.lr = float(h0.reg), float(h0.lr)
+        self.hungarian, self.alpha = False, 0.0
+        self.n_shared = self.dim * self.k + self.dim
+        ids = sorted(sim.nodes)
+        self.data, self.off, self.cnt = self._concat([_np(sim.nodes[i].data[0]).reshape(-1, 2) for i in ids], 2, self.device)
+        self.te, self.te_off, self.te_cnt = self._concat(
+            [_np(sim.nodes[i].data[1]).reshape(-1, 2) if sim.nodes[i].data[1] is not None else np.zeros((0, 2))
+             for i in ids], 2, self.device)
+        self.te_cnt_host = self.te_cnt.cpu().numpy()
+
+    def _deliver_cuda(self, recvs: torch.Tensor, slots: torch.Tensor) -> None:
+        from ..ops.native import native
+        native().mf_bank_deliver(*self._args(), recvs, slots)
+
+    def _parts(self, w: torch.Tensor):
+        m, k = self.dim, self.k
+        return (w[:, :m * k].view(-1, m, k), w[:, m * k:m * k + m], w[:, m * k + m:m * k + m + k],
+                w[:, m * k + m + k])
+
+    def _update_cpu(self, w: torch.Tensor, nodes: torch.Tensor) -> torch.Tensor:
+        """In place on the rows ``w`` [B, Dp]: step i of every node's sequential pass at once (``torch_ref.mf_update``:
+        fp32 arithmetic, the step ``lr * err`` rounded to fp32); returns the age increments."""
+        Y, c, X, b = self._parts(w)
+        cnt, off = self.cnt[nodes].long(), self.off[nodes]
+        dec = float(np.float32(1.0 - self.reg * self.lr))
+        for i in range(int(cnt.max()) if cnt.numel() else 0):
+            L = torch.nonzero(cnt > i).squeeze(1)
+            rat = self.data[off[L] + i]
+            items, r = rat[:, 0].long(), rat[:, 1]
+            yi, xl = Y[L, items], X[L]
+            err = r - (xl * yi).sum(1) - b[L] - c[L, items]
+            step = (err.double() * self.lr).float()
+            yn = yi * dec + step[:, None] * xl
+            X[L] = xl * dec + step[:, None] * yn
+            Y[L, items] = yn
+            b[L] += step
+            c[L, items] += step
+        return cnt
+
+    def _merge_cpu(self, w: torch.Tensor, sv: torch.Tensor, aw: torch.Tensor, asn: torch.Tensor) -> None:
+        den = 2.0 * (aw + asn).double()
+        wa, wb = (aw.double() / den).float()[:, None], (asn.double() / den).float()[:, None]
+        ns = self.n_shared
+        w[:, :ns] = w[:, :ns] * wa + sv[:, :ns] * wb
+
+    def _evaluate(self, nodes: List[int]) -> List[Dict[str, float]]:
+        cnt = self.te_cnt_host
+        if self.device.type == "cuda":
+            from ..ops.native import native
+            sse = native().mf_bank_eval(*self._args(), self._idx(nodes), self.te, self.te_off, self.te_cnt)
+            ops._count()
+            sse = sse.cpu().numpy().astype(np.float64)
+            with np.errstate(divide="ignore", invalid="ignore"):
+                return [{"rmse": float(np.sqrt(s / cnt[i]))} for s, i in zip(sse, nodes)]
+        out = []
+        for i in nodes:                                       # MFModelHandler.evaluate_async, node by node
+            Y, c, X, b = self._parts(self.W[i:i + 1])
+            o = int(self.te_off[i])
+            r = self.te[o:o + int(cnt[i])]
+            idx = r[:, 0].long()
+            pred = Y[0][idx] @ X[0] + b[0:1] + c[0][idx]
+            out.append({"rmse": float(torch.sqrt(torch.mean((r[:, 1] - pred) ** 2)))})
+        return out

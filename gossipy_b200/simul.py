@@ -710,7 +710,7 @@ class GossipSimulator(SimulationEventSender):
                                                "rows": torch.stack(rows)}
         return True
 
-    # native engine: execute bankable set-ups (linear learners) many nodes per launch.  "auto" = on a GPU, or from
+    # native engine: execute bankable set-ups (linear learners, k-means, MF) many nodes per launch.  "auto" = on a GPU, or from
     # 512 nodes on the CPU (where the bank's vectorised-over-nodes update loses to per-node calls for a few big shards)
     batched: Any = "auto"
     native_executor = True    # native engine: eligible set-ups are enqueued from C++ (engine/stream_exec.py);
@@ -774,12 +774,13 @@ class GossipSimulator(SimulationEventSender):
         self.notify_end()
 
     def _run_native_banked(self, sch, n_rounds: int, C) -> None:
-        """Rounds of a bankable simulation: the scheduler's event list of a round is executed by
-        ``engine.bank.LinearBank`` with one kernel launch per phase of a tick."""
-        from .engine.bank import LinearBank
+        """Rounds of a bankable simulation: the scheduler's event list of a round is executed by a bank
+        (``engine.bank.make_bank``: linear learners, k-means or matrix factorisation) with one kernel launch per
+        phase of a tick."""
+        from .engine.bank import make_bank
         bank = self.__dict__.get("_bank")
         if bank is None:
-            bank = self.__dict__["_bank"] = LinearBank(self)
+            bank = self.__dict__["_bank"] = make_bank(self)
             inflight = self.__dict__.pop("_bank_inflight", None)
             if inflight is not None:
                 bank.import_inflight(inflight)
@@ -809,7 +810,8 @@ class GossipSimulator(SimulationEventSender):
                             r.update_message(True)
                 if evals:
                     with nvtx_range("evaluate"):
-                        self.notify_evaluation(t_last, False, bank.evaluate(evals))
+                        # per-node test sets (matrix factorisation) are per-user results, as in _evaluate_nodes
+                        self.notify_evaluation(t_last, bank.eval_on_user, bank.evaluate(evals))
                 self._clock = int(sch.clock)
                 self.notify_timestep(t_last)
         except KeyboardInterrupt:
